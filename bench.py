@@ -201,6 +201,39 @@ def desync(env, acts, gen, preroll):
     return n
 
 
+DUMP_NAMES = ("obs", "reward", "done", "terminal_obs")  # what BatchedUltrasound.step returns, in that order
+DUMP_MAX_BYTES = 64 << 20
+
+
+def dump_outputs(dirname, outputs, world, rank):
+    """Write what the last timed step returned as float32 DIR/<name>.npy (rows of all ranks, in global env order), so that two
+    builds can be compared output for output.  Above DUMP_MAX_BYTES a fixed, seeded sample of env rows is written, with its global
+    env ids in DIR/env_index.npy."""
+    import torch
+    import torch.distributed as dist
+
+    arrays = {}
+    for name, t in zip(DUMP_NAMES, outputs):
+        t = t.float()
+        if world > 1:
+            parts = [torch.empty_like(t) for _ in range(world)]
+            dist.all_gather(parts, t)
+            t = torch.cat(parts)
+        arrays[name] = t.cpu().numpy()
+    if rank != 0:
+        return
+    n = len(arrays["obs"])
+    row_bytes = sum(a[:1].nbytes for a in arrays.values())
+    if n * row_bytes > DUMP_MAX_BYTES:
+        k = (DUMP_MAX_BYTES - 4096) // (row_bytes + 8)  # (4 KiB: the .npy headers)
+        rows = np.sort(np.random.default_rng(SEED).choice(n, size=k, replace=False))
+        arrays = {name: a[rows] for name, a in arrays.items()}
+        arrays["env_index"] = rows.astype(np.float64)
+    os.makedirs(dirname, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(dirname, name + ".npy"), a)
+
+
 def run_cuda(args):
     import torch
     import torch.distributed as dist
@@ -247,12 +280,14 @@ def run_cuda(args):
         if flush is not None:
             flush.zero_()
         evs[i][0].record()
-        env.step(acts[i % nact])
+        last = env.step(acts[i % nact])
         evs[i][1].record()
     barrier()
     t_wall = time.perf_counter() - t_wall
     launches = env.launch_count - l0
     clocks = sampler.result()
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, last, world, rank)
     ms = sum(a.elapsed_time(b) for a, b in evs)
     kms, kn = env.kernel_time(reset=True)
     env.set_timing(False)
@@ -488,7 +523,13 @@ def main():
     ap.add_argument("--no-strong-ref", action="store_true", help="N>1: skip the 1-GPU x all-envs reference measurement on rank 0")
     ap.add_argument("--cpu-steps", type=int, default=0, help="env steps per host thread of the cpu_baseline sample (0: ~15 s of CPU work)")
     ap.add_argument("--traffic", type=float, default=None, help="dram bytes per launch of the dominant kernel from an ncu capture")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="env workload: write what the last timed step returned (obs, reward, done, terminal_obs) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "cuda" or args.workload != "env"):
+        ap.error("--dump-outputs applies to the CUDA env-step workload")
     if args.early_termination:
         ENV_OPTS["early_termination"] = True
     if args.impl == "reference":

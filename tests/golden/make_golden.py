@@ -1,8 +1,8 @@
 #!/usr/bin/env python
 """Generate the golden vectors under tests/golden/ by EXECUTING the reference's own Python.
 
-Runs only in the build container (needs /root/reference, which never travels to the GPU box); the JSON
-files it writes are committed.  What is executed unmodified from the reference checkout:
+Needs a checkout of the reference, named by the RUI_REFERENCE environment variable; the JSON files it
+writes are committed, so the tests never need the reference.  What is executed unmodified from the reference checkout:
 
   * src/utils/quaternion.py ............ q_log, difference_quat, distance_quat
   * src/my_environments/ultrasound.py .. Ultrasound.__init__ constants, reward, _post_action,
@@ -15,7 +15,7 @@ restates documented upstream behaviour [EXT-recall]; everything in the reference
 
 Also decodes the statistics shipped in src/trained_rl_models/ (SURVEY.md App. D) into art_stats.json.
 
-  python tests/golden/make_golden.py
+  RUI_REFERENCE=<checkout> python tests/golden/make_golden.py
 """
 import base64
 import importlib.util
@@ -30,7 +30,7 @@ import zipfile
 
 import numpy as np
 
-REF = "/root/reference/src"
+REF = os.path.join(os.environ["RUI_REFERENCE"], "src")
 OUT = os.path.dirname(os.path.abspath(__file__))
 
 

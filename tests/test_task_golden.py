@@ -172,8 +172,8 @@ def test_oracle_step_returns_the_observation_reward_was_computed_from(O, soft_mo
 def test_scene_params_match_the_reference_mjcf():
     """SceneParams (what the kernels are compiled against) vs the reference's in-tree MJCF (soft_box.xml, soft_human_torso.xml,
     ultrasound_arena.xml + ultrasound_arena.py placement, ultrasound_probe_gripper.xml), parsed by the package's own reader.  The
-    committed parse (tests/golden/mjcf_golden.json, written by make_golden.py) is checked always; where the reference checkout is
-    present the files are re-read and must give the same parse."""
+    committed parse (tests/golden/mjcf_golden.json, written by make_golden.py) is checked always; where RUI_REFERENCE names a
+    checkout of the reference the files are re-read and must give the same parse."""
     import json
     import os
 
@@ -190,8 +190,8 @@ def test_scene_params_match_the_reference_mjcf():
         assert mjcf.check_scene_params(params, gold[key]) == {}, key
         f = mjcf.scene_fields(gold[key])
         assert f["comp_count"] == (9, 4, 11) and f["solref_smooth"] == (-1324.17, -17.59) and f["probe_pos"] == (-0.004, -0.063, 0.128)
-        ref = "/root/reference/src/my_models"
-        if os.path.isdir(ref):
+        if os.environ.get("RUI_REFERENCE"):
+            ref = os.path.join(os.environ["RUI_REFERENCE"], "src", "my_models")
             assert norm(mjcf.read_assets(ref, box)) == gold[key]
             assert mjcf.scene_params_from_mjcf(ref, box) == params
     # a deliberately wrong constant is caught
