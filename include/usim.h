@@ -201,6 +201,27 @@ int usim_set_state(usim_handle* h, const float* qpos_dev, const float* qvel_dev,
 int usim_get_contacts(usim_handle* h, int32_t* ncon_dev, int32_t* geom1_dev, int32_t* geom2_dev,
                       float* dist_dev, void* stream);
 
+/* Contact record, opt-in.  enable != 0 turns it on for the launches issued after
+ * this call (the record is allocated on the first enable: USIM_MAX_CONTACTS * 36
+ * bytes per env); with it off every launch runs exactly as without it. */
+int usim_set_contact_record(usim_handle* h, int enable);
+
+/* Position, frame and constraint force of every contact of the last forward
+ * pass -- the same pass usim_get_contacts and usim_get_diag describe, contact c
+ * being row c of their list.  Replaces `sim.data.contact[:ncon].pos / .frame`
+ * and `mujoco_py.functions.mj_contactForce(model, data, c, f)` (its first three
+ * components: condim 3).  Device memory:
+ *   pos_dev   [num_envs][USIM_MAX_CONTACTS][3] float, world contact point
+ *   frame_dev [num_envs][USIM_MAX_CONTACTS][9] float, rows: the normal (geom1 ->
+ *             geom2), then two tangents (MuJoCo's rule)
+ *   force_dev [num_envs][USIM_MAX_CONTACTS][3] float, (normal, tangent 1,
+ *             tangent 2) force on geom2 in that frame; frame^T force is the
+ *             world force, and the forces on the probe add up to diag[0..2]
+ * Rows at or beyond ncon are zero; any pointer may be NULL.  Fails unless
+ * recording is on and every env has been stepped (or reset without mask) since
+ * it was last enabled.  A diverged env reports zero forces. */
+int usim_get_contact_forces(usim_handle* h, float* pos_dev, float* frame_dev, float* force_dev, void* stream);
+
 /* Per-env diagnostics of the last step, [num_envs][USIM_DIAG_DIM] float:
  * 0-2 cfrc_ext[probe][-3:] (ultrasound.py:365), 3-5 ee torque (:369),
  * 6-8 eef pos, 9-12 eef quat xyzw, 13-19 joint torques, 20 solver iterations,

@@ -27,6 +27,8 @@ SYMBOLS = {
     "usim_set_state": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _vp]),
     "usim_get_contacts": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _vp]),
     "usim_get_diag": (C.c_int, [_vp, _vp, _vp]),
+    "usim_set_contact_record": (C.c_int, [_vp, C.c_int]),
+    "usim_get_contact_forces": (C.c_int, [_vp, _vp, _vp, _vp, _vp]),
     "usim_get_arm_record": (C.c_int, [_vp, _vp, _vp]),
     "usim_num_envs": (C.c_int, [_vp]),
     "usim_nq": (C.c_int, [_vp]),

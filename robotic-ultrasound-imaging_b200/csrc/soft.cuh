@@ -375,7 +375,32 @@ struct SolveArgs {
   const int *prep_items, *prep_n;  // prepare mode: the requests this launch works through
   unsigned long long* trace;       // developer trace (USIM_TRACE): per env (start ns, end ns, SM id) of the launch, nullptr: off
   int* queue;                      // persistent launch (grid = resident CTAs): next launch slot, fetched with atomicAdd (nullptr: item = blockIdx.x + k gridDim.x)
+  float* crec_out;                 // contact record [n][DEV_MAXC][CREC_DIM] (rows c < ncon), nullptr: recording off (usim_set_contact_record)
 };
+// one contact of the record: point (world), normal (geom1 -> geom2), world force on geom2 -- usim_get_contact_forces turns it into
+// MuJoCo's contact frame and frame-coordinate force
+#define CREC_DIM 9
+
+// Contact record of one env (rows c < ncon): point, normal, cone_force of the final j -- every exit of the CG loop follows an
+// update_grad on the final cjar (the line search moves cjar right before it), so these are the forces the probe wrench was summed
+// from.  Runs after K9 and reads only shared memory; not inlined, so that the solve kernel's register allocation and schedule (the CG
+// loop instruction for instruction) stay those of the kernel without the record.  A diverged env records zero forces, as K9 zeroes
+// its cfrc: a non-finite solution (the x norm of the divergence guard, in rq) or probe wrench -- a non-finite arm state ends up in both.
+__device__ __noinline__ void record_contacts(const WS& w, float* rec, int ncon, int tid) {
+  const bool zero = !isfinite(rd(w.rq, 0)) || !isfinite(rd(w.rg, 6) + rd(w.rg, 7) + rd(w.rg, 8));
+#pragma unroll 1
+  for (int c = tid; c < ncon; c += NT) {
+    int zone;
+    float fr, mu, Dn = w.cD[c];
+    contact_params(w.ctype[c], fr, mu);
+    const v3 nn = mk(w.cn[0][c], w.cn[1][c], w.cn[2][c]);
+    const v3 Fw = zero ? mk(0, 0, 0) : cone_force(mk(w.cjar[0][c], w.cjar[1][c], w.cjar[2][c]), nn, Dn, Dn * dm.impratio, mu, fr, zone);
+    float* r = rec + (size_t)c * CREC_DIM;
+    r[0] = w.cpos[0][c]; r[1] = w.cpos[1][c]; r[2] = w.cpos[2][c];
+    r[3] = nn.x; r[4] = nn.y; r[5] = nn.z;
+    r[6] = Fw.x; r[7] = Fw.y; r[8] = Fw.z;
+  }
+}
 
 __global__ void __launch_bounds__(NT, MINB) solve_kernel(const SolveArgs a) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
@@ -1551,6 +1576,8 @@ __global__ void __launch_bounds__(NT, MINB) solve_kernel(const SolveArgs a) {
     a.bin_items[(size_t)b * n + atomicAdd(a.bin_cnt + b, 1)] = env;
   }
   env_sync();
+  // ------------------------------------------------------------------ contact record (opt-in, usim_set_contact_record)
+  if (a.crec_out) record_contacts(w, a.crec_out + (size_t)env * DEV_MAXC * CREC_DIM, ncon, tid);
   if (mode != 2 && tid < USIM_OBS_DIM) { // this step's observation: the terminal one if a prepared reset state takes over below
     float* o = w.consume ? (a.tobs ? a.tobs + (size_t)env * USIM_OBS_DIM : nullptr) : obs_row;
     if (o) o[tid] = w.orow[tid];

@@ -38,6 +38,10 @@ struct usim_handle {
   float *qpos = nullptr, *qvel = nullptr, *warm = nullptr, *task = nullptr, *armbuf = nullptr, *diag = nullptr;
   int *ncon = nullptr, *geom1 = nullptr, *geom2 = nullptr;
   float* cdist = nullptr;
+  // contact record (usim_set_contact_record): [n][DEV_MAXC][CREC_DIM], allocated on the first enable; complete once every env has
+  // been through a recorded launch (a step, or a reset without mask)
+  float* crec = nullptr;
+  bool crec_on = false, crec_complete = false;
   int* counters = nullptr; // [0] env steps that produced a non-finite solution (episode force-ended), [1] env steps whose contact list overflowed
   // model tables
   float4 *ax4 = nullptr, *ps4 = nullptr; // (axis, dof_invweight0), (rest position, body_invweight0)
@@ -317,7 +321,7 @@ int usim_destroy(usim_handle* h) {
     cudaFree(h->trace);
   }
   for (auto& p : h->pending) { cudaEventDestroy(p.first); cudaEventDestroy(p.second); }
-  void* dev[] = {h->counters, h->qpos, h->qvel, h->warm, h->task, h->armbuf, h->diag, h->ncon, h->geom1, h->geom2, h->cdist, h->ax4,
+  void* dev[] = {h->counters, h->qpos, h->qvel, h->warm, h->task, h->armbuf, h->diag, h->ncon, h->geom1, h->geom2, h->cdist, h->crec, h->ax4,
                  h->ps4, h->nb4, h->eq_pairs, h->d_act, h->d_obs, h->d_tobs, h->d_rew,
                  h->d_done, h->d_resetmask, h->bin_cnt, h->bin_items, h->order, h->queue, h->slot_qpos, h->slot_task, h->slot_obs, h->prep_armbuf,
                  h->req_list, h->req_cnt};
@@ -382,6 +386,7 @@ static SolveArgs base_args(usim_handle* h, int mode) {
   a.pt = tables(h); a.eq_pairs = h->eq_pairs;
   a.diag = h->diag; a.ncon_out = h->ncon; a.geom1_out = h->geom1; a.geom2_out = h->geom2; a.dist_out = h->cdist;
   a.counters = h->counters;
+  a.crec_out = h->crec_on && mode != 2 ? h->crec : nullptr; // an intermediate substep's contacts are superseded by the last one's
   a.slot_qpos = h->slot_qpos; a.slot_task = h->slot_task; a.slot_obs = h->slot_obs;
   return a;
 }
@@ -405,7 +410,7 @@ static int producer_end(usim_handle* h, cudaStream_t s) {
   RESET_LAUNCH(h, 64, 32, h->prep_stream, n, nullptr, h->slot_qpos, nullptr, nullptr, h->slot_task, h->prep_armbuf, list, cnt, nullptr, nullptr);
   SolveArgs a = base_args(h, 1);
   a.prep = 1; a.armbuf = h->prep_armbuf; a.prep_items = list; a.prep_n = cnt;
-  a.diag = nullptr; a.ncon_out = nullptr; a.geom1_out = nullptr; a.geom2_out = nullptr; a.dist_out = nullptr;
+  a.diag = nullptr; a.ncon_out = nullptr; a.geom1_out = nullptr; a.geom2_out = nullptr; a.dist_out = nullptr; a.crec_out = nullptr;
   solve_kernel<<<PREP_GRID, NT, h->smem, h->prep_stream>>>(a);
   CK(cudaMemsetAsync(cnt, 0, sizeof(int), h->prep_stream));
   CK(cudaEventRecord(h->ev_prep[b], h->prep_stream));
@@ -452,6 +457,7 @@ static int launch_step(usim_handle* h, const float* act, float* obs, float* rew,
     h->solve_tick += 1;
     if (last && auto_reset && producer_end(h, s)) return -1;
   }
+  if (h->crec_on) h->crec_complete = true;
   CK(cudaGetLastError());
   return 0;
 }
@@ -478,6 +484,7 @@ int usim_reset(usim_handle* h, const uint8_t* mask_dev, float* obs_dev, void* st
   solve_kernel<<<n, NT, h->smem, s>>>(a);
   h->launches += 2;
   CK(cudaGetLastError());
+  if (h->crec_on && !mask_dev) h->crec_complete = true;
   if (producer_end(h, s)) return -1;
   return mark_state(h, s);
 }
@@ -626,6 +633,54 @@ int usim_get_contacts(usim_handle* h, int32_t* ncon, int32_t* g1, int32_t* g2, f
   if (g1) CK(cudaMemcpyAsync(g1, h->geom1, N * DEV_MAXC * sizeof(int), cudaMemcpyDeviceToDevice, s));
   if (g2) CK(cudaMemcpyAsync(g2, h->geom2, N * DEV_MAXC * sizeof(int), cudaMemcpyDeviceToDevice, s));
   if (dist) CK(cudaMemcpyAsync(dist, h->cdist, N * DEV_MAXC * sizeof(float), cudaMemcpyDeviceToDevice, s));
+  return 0;
+}
+int usim_set_contact_record(usim_handle* h, int enable) {
+  if (!h) return fail("usim_set_contact_record: null handle");
+  if (enable && !h->crec) {
+    CK(cudaSetDevice(h->device));
+    CK(cudaMalloc((void**)&h->crec, (size_t)h->n * DEV_MAXC * CREC_DIM * sizeof(float)));
+  }
+  if (!enable || !h->crec_on) h->crec_complete = false; // the record no longer follows the contact list until every env is launched again
+  h->crec_on = enable != 0;
+  return 0;
+}
+
+// record row -> MuJoCo layouts: contact frame (rows: normal, then the tangents of the make_frame rule: the world y axis, or z when the
+// normal is within 60 degrees of y, orthogonalised against the normal; third = normal x second) and the force in that frame
+__global__ void contact_forces_kernel(int n, const int* __restrict__ ncon, const float* __restrict__ rec, float* __restrict__ pos,
+                                      float* __restrict__ frame, float* __restrict__ force) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n * DEV_MAXC) return;
+  const int c = i % DEV_MAXC;
+  float p[3] = {0, 0, 0}, fm[9] = {0, 0, 0, 0, 0, 0, 0, 0, 0}, f[3] = {0, 0, 0};
+  if (c < ncon[i / DEV_MAXC]) {
+    const float* r = rec + (size_t)i * CREC_DIM;
+    const v3 nn = mk(r[3], r[4], r[5]), F = mk(r[6], r[7], r[8]);
+    const v3 t = fabsf(nn.y) < 0.5f ? mk(0, 1, 0) : mk(0, 0, 1);
+    v3 y = t - dot(nn, t) * nn;
+    y = (1.f / norm(y)) * y;
+    const v3 z = cross(nn, y);
+    p[0] = r[0]; p[1] = r[1]; p[2] = r[2];
+    fm[0] = nn.x; fm[1] = nn.y; fm[2] = nn.z; fm[3] = y.x; fm[4] = y.y; fm[5] = y.z; fm[6] = z.x; fm[7] = z.y; fm[8] = z.z;
+    f[0] = dot(nn, F); f[1] = dot(y, F); f[2] = dot(z, F);
+  }
+  if (pos) for (int k = 0; k < 3; k++) pos[(size_t)i * 3 + k] = p[k];
+  if (frame) for (int k = 0; k < 9; k++) frame[(size_t)i * 9 + k] = fm[k];
+  if (force) for (int k = 0; k < 3; k++) force[(size_t)i * 3 + k] = f[k];
+}
+
+int usim_get_contact_forces(usim_handle* h, float* pos, float* frame, float* force, void* stream) {
+  if (!h) return fail("usim_get_contact_forces: null handle");
+  if (!h->crec) return fail("usim_get_contact_forces: contact recording was never enabled (usim_set_contact_record)");
+  if (!h->crec_complete)
+    return fail("usim_get_contact_forces: no step or reset of every env has run since contact recording was enabled");
+  if (!pos && !frame && !force) return 0;
+  CK(cudaSetDevice(h->device));
+  const int tot = h->n * DEV_MAXC;
+  contact_forces_kernel<<<(tot + 255) / 256, 256, 0, (cudaStream_t)stream>>>(h->n, h->ncon, h->crec, pos, frame, force);
+  h->launches += 1;
+  CK(cudaGetLastError());
   return 0;
 }
 int usim_get_diag(usim_handle* h, float* diag, void* stream) {

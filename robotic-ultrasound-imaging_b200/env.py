@@ -85,6 +85,7 @@ class BatchedUltrasound:
         solver_iterations: int = 40,
         solver_tolerance: float = 3e-5,
         scene_params: Optional[SceneParams] = None,
+        record_contacts: bool = False,
         **cfg_kwargs,
     ):
         if not torch.cuda.is_available():
@@ -111,6 +112,8 @@ class BatchedUltrasound:
         self.term_obs = torch.zeros(N, OBS_DIM, device=dev)
         self.rew = torch.zeros(N, device=dev)
         self.done = torch.zeros(N, dtype=torch.uint8, device=dev)
+        if record_contacts:
+            self.set_contact_record(True)
 
     # -- lifecycle ---------------------------------------------------------
     def close(self):
@@ -192,6 +195,23 @@ class BatchedUltrasound:
         with torch.cuda.device(self.device):
             _lib.check(_lib.lib().usim_get_contacts(self._h, _ptr(ncon), _ptr(g1), _ptr(g2), _ptr(dist), self._stream()))
         return ncon, g1, g2, dist
+
+    def set_contact_record(self, enable: bool = True):
+        """Record position, frame and force of every contact from the next step / reset on (read with :meth:`contact_forces`).
+        Off by default: the record costs one store pass over the contacts per step and USIM_MAX_CONTACTS * 36 bytes per env."""
+        _lib.check(_lib.lib().usim_set_contact_record(self._h, int(enable)))
+
+    def contact_forces(self):
+        """``sim.data.contact[:ncon].pos / .frame`` and ``mj_contactForce`` of the last forward pass (the one :meth:`contacts`
+        lists): pos [N, MAX_CONTACTS, 3], frame [N, MAX_CONTACTS, 3, 3] (rows: normal geom1 -> geom2, two tangents) and force
+        [N, MAX_CONTACTS, 3] on geom2 in that frame (normal, tangent 1, tangent 2).  Rows at or beyond ncon are zero."""
+        N, dev = self.num_envs, self.device
+        pos = torch.empty(N, MAX_CONTACTS, 3, device=dev)
+        frame = torch.empty(N, MAX_CONTACTS, 3, 3, device=dev)
+        force = torch.empty(N, MAX_CONTACTS, 3, device=dev)
+        with torch.cuda.device(self.device):
+            _lib.check(_lib.lib().usim_get_contact_forces(self._h, _ptr(pos), _ptr(frame), _ptr(force), self._stream()))
+        return pos, frame, force
 
     def diag(self):
         d = torch.empty(self.num_envs, DIAG_DIM, device=self.device)
@@ -421,7 +441,7 @@ class Ultrasound:
             1, device=device, soft_torso=soft_torso, controller_configs=controller_configs, control_freq=control_freq,
             horizon=horizon, early_termination=early_termination, torso_solref_randomization=torso_solref_randomization,
             initial_probe_pos_randomization=initial_probe_pos_randomization, deterministic_trajectory=deterministic_trajectory,
-            seed=seed, ignore_done=ignore_done, scene_params=scene_params)
+            seed=seed, ignore_done=ignore_done, scene_params=scene_params, record_contacts=True)
         self.robots = [_Robot(self)]
         self.timestep = 0
         self.done = True
@@ -552,6 +572,18 @@ class Ultrasound:
             if (nx in a and (b is None or ny in b)) or (ny in a and (b is None or nx in b)):
                 return True
         return False
+
+    def get_contacts(self) -> List[Dict[str, Any]]:
+        """The active contacts of the last forward pass, as a mujoco-py user reads them: for each of ``sim.data.contact[:ncon]``
+        the geom names, ``dist``, ``pos``, ``frame`` (3x3, rows: normal geom1 -> geom2, two tangents) and ``force``, the
+        first three components of ``mj_contactForce`` (normal, tangent 1, tangent 2: the force on geom2 in that frame)."""
+        ncon, g1, g2, dist = self.core.contacts()
+        pos, frame, force = self.core.contact_forces()
+        n, m = int(ncon[0].item()), self.core.model
+        g1, g2, dist = g1[0, :n].tolist(), g2[0, :n].tolist(), dist[0, :n].cpu().numpy().astype(np.float64)
+        pos, frame, force = [x[0, :n].cpu().numpy().astype(np.float64) for x in (pos, frame, force)]
+        return [dict(geom1=m.geom_name(g1[c]), geom2=m.geom_name(g2[c]), dist=float(dist[c]), pos=pos[c], frame=frame[c], force=force[c])
+                for c in range(n)]
 
     def _check_probe_contact_with_table(self) -> bool:
         """ultrasound.py:739-746"""

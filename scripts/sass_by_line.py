@@ -44,6 +44,9 @@ def region(line):
 
 cnt, per_line = collections.Counter(), collections.Counter()
 cur_file, cur_line, in_k, total = None, 0, False, 0
+# the CG loop: from the target of its back edge (a branch attributed to the K6 `for` statement) to that branch
+cg_line = next(i for i, l in enumerate(src, 1) if "for (int it = -1; it < maxit; it++)" in l)
+labels, back = {}, []
 for l in sass.splitlines():
     if ".section" in l and ".text." in l:
         in_k = kernel in l
@@ -53,12 +56,20 @@ for l in sass.splitlines():
     if m:
         cur_file, cur_line = os.path.basename(m.group(1)), int(m.group(2))
         continue
+    m = re.match(r"^\s*(\.L_x_\d+):", l)
+    if m:
+        labels[m.group(1)] = total
+    m = re.search(r"BRA.*\(\s*(\.L_x_\d+)\s*\)", l)
+    if m and cur_file == "soft.cuh" and cur_line == cg_line and m.group(1) in labels:
+        back.append(total - labels[m.group(1)] + 1)
     if re.match(r"\s+/\*[0-9a-f]{4,6}\*/", l):
         total += 1
         key = region(cur_line) if cur_file == "soft.cuh" else cur_file
         cnt[key] += 1
         per_line[(cur_file, cur_line)] += 1
 print(f"{kernel}: {total} SASS instructions ({total * 16 / 1024:.0f} KB)")
+if back:
+    print(f"CG loop (soft.cuh:{cg_line}): {max(back)} SASS instructions")
 for k, v in cnt.most_common():
     print(f"{v:6d}  {k}")
 print("top lines:")
