@@ -187,7 +187,17 @@ int usim_step_host(usim_handle* h, const float* act_host, float* obs_host, float
 
 /* State access, parity hooks.  Replace `sim.data.qpos/qvel/qacc_warmstart`
  * views and `sim.data.set_joint_qpos` (ultrasound.py:430).  Layout
- * [num_envs][nq|nv|USIM_TASK_DIM] float, device memory. */
+ * [num_envs][nq|nv|USIM_TASK_DIM] float, device memory.
+ * usim_set_state with a task record, once usim_reset has run, also prepares
+ * again (on `stream`, the next call on it waits for this) the reset states the
+ * next two auto-resets of every env take over: episodes E and E + 1, E being
+ * the restored USIM_TS_EPISODE.  So an auto-reset after a restore draws what the
+ * (seed, global env id, episode) streams give for the restored counter, as
+ * usim_reset does.  The arm record is not part of the state, and the solver's
+ * warm start is shifted by the change of the arm's qfrc_smooth since the
+ * previous step, which it holds: until its next reset a restored env agrees
+ * with the run it was saved from to solver tolerance, from then on bit for bit
+ * (a reset state starts from a zero warm start, without shift). */
 int usim_get_state(usim_handle* h, float* qpos_dev, float* qvel_dev, float* warm_dev, float* task_dev, void* stream);
 int usim_set_state(usim_handle* h, const float* qpos_dev, const float* qvel_dev, const float* warm_dev,
                    const float* task_dev, void* stream);

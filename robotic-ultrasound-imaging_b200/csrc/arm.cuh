@@ -525,11 +525,14 @@ __global__ void __launch_bounds__(32) reset_kernel(int n, const uint8_t* __restr
   } // work items
 }
 
-// first reset of a handle: request the two episodes that follow the first one (numbers 1 and 2) for EVERY env
-__global__ void fill_requests_kernel(int n, int* __restrict__ req_list, int* __restrict__ req_cnt) {
+// Fill both slots of EVERY env: request episode numbers E and E + 1, E = the counter of the env's live task record (the reset
+// states its next two auto-resets take over).  Runs after the first reset of a handle (no slot prepared yet) and after
+// usim_set_state (the restored counters need not be those the slots were prepared for).
+__global__ void fill_requests_kernel(int n, const float* __restrict__ task, int* __restrict__ req_list, int* __restrict__ req_cnt) {
   const int env = blockIdx.x * blockDim.x + threadIdx.x;
   if (env >= n) return;
+  const int E = (int)task[(size_t)env * USIM_TASK_DIM + USIM_TS_EPISODE];
   const int p = atomicAdd(req_cnt, 2);
-  req_list[2 * p] = env; req_list[2 * p + 1] = 1;
-  req_list[2 * p + 2] = env; req_list[2 * p + 3] = 2;
+  req_list[2 * p] = env; req_list[2 * p + 1] = E;
+  req_list[2 * p + 2] = env; req_list[2 * p + 3] = E + 1;
 }

@@ -421,6 +421,19 @@ static int producer_end(usim_handle* h, cudaStream_t s) {
   return 0;
 }
 
+// A producer of its own that fills both slots of every env from its live episode counter (fill_requests_kernel).  Stream s then
+// waits for the prepare run: the very next step may end an episode and take over either slot, whereas producer_begin orders a step
+// only after the slots filled two producers before it.
+static int prepare_slots(usim_handle* h, cudaStream_t s) {
+  const int b = (int)(h->prod_tick & 1), n = h->n;
+  if (producer_begin(h, s)) return -1;
+  fill_requests_kernel<<<(n + 127) / 128, 128, 0, s>>>(n, h->task, h->req_list + (size_t)b * 2 * 3 * n, h->req_cnt + b);
+  h->launches += 1;
+  if (producer_end(h, s)) return -1;
+  CK(cudaStreamWaitEvent(s, h->ev_prep[b], 0));
+  return 0;
+}
+
 // One control step: int(control_timestep / timestep) physics substeps of (arm kernel, solve kernel); the OSC goal is set on the
 // first substep, the task epilogue -- and, with auto_reset, the hand-over to a prepared reset state -- runs in the last solve launch
 // [robosuite MujocoEnv.step].
@@ -467,25 +480,27 @@ int usim_reset(usim_handle* h, const uint8_t* mask_dev, float* obs_dev, void* st
   if (activate(h)) return -1;
   cudaStream_t s = (cudaStream_t)stream;
   const int n = h->n;
-  if (producer_begin(h, s)) return -1;
-  int* list = h->req_list + (size_t)(h->prod_tick & 1) * 2 * 3 * n;
-  int* cnt = h->req_cnt + (h->prod_tick & 1);
   const bool first = !h->slots_init;
-  if (first) { // nothing prepared yet: the two episodes after the first one, for every env (all episode counters are 0 here)
-    fill_requests_kernel<<<(n + 127) / 128, 128, 0, s>>>(n, list, cnt);
-    h->slots_init = true;
-    h->launches += 1;
+  int *list = nullptr, *cnt = nullptr;
+  if (!first) { // the live reset of an env with counter E files a request for episode E + 2 (the slot of E is stale from here on)
+    if (producer_begin(h, s)) return -1;
+    list = h->req_list + (size_t)(h->prod_tick & 1) * 2 * 3 * n;
+    cnt = h->req_cnt + (h->prod_tick & 1);
   }
   // the reset itself, in place and in stream order: reset kernel (live mode) + forward-only solve on the live state
-  RESET_LAUNCH(h, (n + 31) / 32, 32, s, n, mask_dev, h->qpos, h->qvel, h->warm, h->task, h->armbuf, nullptr, nullptr,
-               first ? nullptr : list, first ? nullptr : cnt);
+  RESET_LAUNCH(h, (n + 31) / 32, 32, s, n, mask_dev, h->qpos, h->qvel, h->warm, h->task, h->armbuf, nullptr, nullptr, list, cnt);
   SolveArgs a = base_args(h, 1);
   a.mask = mask_dev; a.obs = obs_dev;
   solve_kernel<<<n, NT, h->smem, s>>>(a);
   h->launches += 2;
   CK(cudaGetLastError());
   if (h->crec_on && !mask_dev) h->crec_complete = true;
-  if (producer_end(h, s)) return -1;
+  if (first) { // nothing prepared yet: both slots of every env, from the counters this reset left
+    h->slots_init = true;
+    if (prepare_slots(h, s)) return -1;
+  } else if (producer_end(h, s)) {
+    return -1;
+  }
   return mark_state(h, s);
 }
 
@@ -615,6 +630,9 @@ int usim_set_state(usim_handle* h, const float* qpos, const float* qvel, const f
   if (warm) rc(h, h->nv, h->nv, QPAD, warm, h->warm, s);
   if (task) rc(h, USIM_TASK_DIM, USIM_TASK_DIM, USIM_TASK_DIM, task, h->task, s);
   CK(cudaGetLastError());
+  // the slots hold the reset states of the counters before the restore: prepare them again from the restored ones (bit-identical
+  // slots where a counter did not change, since a prepared state depends on nothing but (seed, env id, episode number))
+  if (task && h->slots_init && prepare_slots(h, s)) return -1;
   return mark_state(h, s);
 }
 
