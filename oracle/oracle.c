@@ -1074,6 +1074,75 @@ void oracle_forward(oracle_env* e, const double* ctrl) {
   forward_acc(e, ctrl);
 }
 
+/* The problem of the last forward pass (rows, a0, M, J, D, aref) evaluated at a given qacc; the env is left as it was.
+ * rhs and Hx are formed as the device solver forms them: M plus the equality rows (fix, smooth, tendon) is its quadratic part H,
+ *   rhs = qfrc_smooth + sum_eq J^T D aref,   Hx = H qacc - rhs (the kernel's Hx row holds the gradient of the quadratic part),
+ *   grad = Hx - sum_other J^T f = M (qacc - a0) - J^T f,
+ * and its stopping rule is |grad| <= tol (1 + |rhs| + |Hx|): norms[0] = |grad|, norms[1] = |rhs|, norms[2] = |Hx|. */
+int oracle_evaluate(oracle_env* e, const double* qacc, double* grad, double* cost, double* efc_force, double* contact_force,
+                    double* cfrc, double* ft_torque, double* norms) {
+  int nv = e->nv, nefc = e->nefc;
+  double* save_qacc = dalloc(nv);
+  double* save_jar = dalloc(nefc);
+  double* save_frc = dalloc(nefc);
+  double* rhs = dalloc(nv);
+  double* hx = dalloc(nv);
+  double* g = dalloc(nv);
+  double save_force[USIM_MAX_CONTACTS][3], save_cfrc[3], save_ft[3];
+  int save_in_contact = e->in_contact;
+  memcpy(save_qacc, e->qacc, sizeof(double) * nv);
+  memcpy(save_jar, e->jar, sizeof(double) * nefc);
+  memcpy(save_frc, e->frc, sizeof(double) * nefc);
+  for (int c = 0; c < e->ncon; c++) memcpy(save_force[c], e->con[c].force, sizeof save_force[c]);
+  memcpy(save_cfrc, e->cfrc, sizeof save_cfrc);
+  memcpy(save_ft, e->ft_torque, sizeof save_ft);
+
+  memcpy(e->qacc, qacc, sizeof(double) * nv);
+  row_mul(e, qacc, e->jar);
+  for (int r = 0; r < nefc; r++) e->jar[r] -= e->raref[r];
+  double c = constraint_update(e, e->jar, e->frc, NULL);
+  sym_mul(e->M, nv, qacc, hx);
+  memcpy(rhs, e->qs, sizeof(double) * nv);
+  for (int i = 0; i < nv; i++) e->tmp[i] = qacc[i] - e->a0[i];
+  sym_mul(e->M, nv, e->tmp, g);
+  for (int i = 0; i < nv; i++) c += 0.5 * e->tmp[i] * g[i];
+  for (int r = 0; r < nefc; r++) {
+    const int* idx = e->pidx + e->rstart[r];
+    const double* val = e->pval + e->rstart[r];
+    for (int i = 0; i < e->rn[r]; i++) {
+      g[idx[i]] -= val[i] * e->frc[r];
+      if (e->rtype[r] == ROW_EQ) {
+        hx[idx[i]] += val[i] * e->rD[r] * (e->jar[r] + e->raref[r]);
+        rhs[idx[i]] += val[i] * e->rD[r] * e->raref[r];
+      }
+    }
+  }
+  double gn = 0, rn = 0, hn = 0;
+  for (int i = 0; i < nv; i++) { gn += g[i] * g[i]; rn += rhs[i] * rhs[i]; hn += (hx[i] - rhs[i]) * (hx[i] - rhs[i]); }
+  post_constraint(e);
+  if (grad) memcpy(grad, g, sizeof(double) * nv);
+  if (cost) *cost = c;
+  if (efc_force) memcpy(efc_force, e->frc, sizeof(double) * nefc);
+  if (contact_force)
+    for (int k = 0; k < e->ncon; k++) memcpy(contact_force + 3 * k, e->con[k].force, 3 * sizeof(double));
+  if (cfrc) memcpy(cfrc, e->cfrc, sizeof e->cfrc);
+  if (ft_torque) memcpy(ft_torque, e->ft_torque, sizeof e->ft_torque);
+  if (norms) { norms[0] = sqrt(gn); norms[1] = sqrt(rn); norms[2] = sqrt(hn); }
+
+  memcpy(e->qacc, save_qacc, sizeof(double) * nv);
+  memcpy(e->jar, save_jar, sizeof(double) * nefc);
+  memcpy(e->frc, save_frc, sizeof(double) * nefc);
+  for (int k = 0; k < e->ncon; k++) memcpy(e->con[k].force, save_force[k], sizeof save_force[k]);
+  memcpy(e->cfrc, save_cfrc, sizeof save_cfrc);
+  memcpy(e->ft_torque, save_ft, sizeof save_ft);
+  e->in_contact = save_in_contact;
+  free(save_qacc); free(save_jar); free(save_frc); free(rhs); free(hx); free(g);
+  return nefc;
+}
+
+/* row type of every constraint row of the last forward pass: 0 equality, 1 joint limit, 2 contact normal, 100 contact friction */
+void oracle_efc_type(const oracle_env* e, int* type) { memcpy(type, e->rtype, sizeof(int) * e->nefc); }
+
 /* mj_Euler: implicit joint damping, semi-implicit update, quaternion integration */
 static void integrate(oracle_env* e) {
   const usim_model* m = e->m;

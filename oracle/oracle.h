@@ -44,6 +44,16 @@ void oracle_set_state(oracle_env* e, const double* qpos, const double* qvel, con
 /* forward pass at the current state with the given joint torques (no integration) */
 void oracle_forward(oracle_env* e, const double* ctrl7);
 
+/* The problem of the last oracle_forward evaluated at `qacc` (nv), the env left unchanged; any output may be NULL.
+ * grad [nv] = M (qacc - a0) - J^T f, cost = the primal cost, efc_force [nefc] = f of every row, contact_force [3 ncon] as
+ * oracle_contacts, cfrc [3] / ft_torque [3] as diag[0:6], norms [3] = |grad|, |rhs|, |Hx| of the device solver's stopping rule
+ * (its quadratic part H is M plus the equality rows; rhs = qfrc_smooth + the equality
+ * rows' J^T D aref, Hx = H qacc - rhs).  Returns nefc. */
+int oracle_evaluate(oracle_env* e, const double* qacc, double* grad, double* cost, double* efc_force, double* contact_force,
+                    double* cfrc, double* ft_torque, double* norms);
+/* row type of every row of the last forward pass: 0 equality, 1 joint limit, 2 contact normal, 100 contact friction */
+void oracle_efc_type(const oracle_env* e, int* type);
+
 /* introspection of the last forward pass */
 int oracle_ncon(const oracle_env* e);
 void oracle_contacts(const oracle_env* e, int* geom1, int* geom2, double* dist, double* pos, double* frame, double* force);

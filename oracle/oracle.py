@@ -54,6 +54,9 @@ def lib():
         for f in ("oracle_qacc", "oracle_qacc_smooth", "oracle_M", "oracle_bias", "oracle_tau"):
             getattr(L, f).restype = _pd
             getattr(L, f).argtypes = [C.c_void_p]
+        L.oracle_evaluate.restype = C.c_int
+        L.oracle_evaluate.argtypes = [C.c_void_p, _pd, _pd, _pd, _pd, _pd, _pd, _pd, _pd]
+        L.oracle_efc_type.argtypes = [C.c_void_p, _pi]
         L.oracle_diag.argtypes = [C.c_void_p, _pd]
         L.oracle_eef.argtypes = [C.c_void_p, _pd, _pd, _pd]
         L.oracle_controller.argtypes = [C.c_void_p, _pd, _pd]
@@ -185,6 +188,21 @@ class OracleEnv:
         d = np.zeros(DIAG_DIM)
         lib().oracle_diag(self.h, _p(d))
         return d
+
+    def evaluate(self, qacc):
+        """The problem of the last forward() evaluated at ``qacc`` (the env is left unchanged): grad = M (qacc - a0) - J^T f, the
+        primal cost, the force of every constraint row and its type (0 equality, 1 joint limit, 2 contact normal, 100 friction),
+        the contact forces (as contacts()["force"]), cfrc and the F/T torque (as diag()[0:6]), and the norms of the device
+        solver's stopping rule |grad| <= tol (1 + |rhs| + |Hx|)."""
+        a = _f64(qacc, self.nv)
+        nefc, ncon = self.nefc, self.ncon
+        grad, cost, frc = np.zeros(self.nv), C.c_double(), np.zeros(max(nefc, 1))
+        cf, cfrc, ft, norms = np.zeros(3 * max(ncon, 1)), np.zeros(3), np.zeros(3), np.zeros(3)
+        lib().oracle_evaluate(self.h, _p(a), _p(grad), C.byref(cost), _p(frc), _p(cf), _p(cfrc), _p(ft), _p(norms))
+        typ = np.zeros(max(nefc, 1), np.intc)
+        lib().oracle_efc_type(self.h, typ.ctypes.data_as(_pi))
+        return dict(grad=grad, cost=cost.value, efc_force=frc[:nefc], efc_type=typ[:nefc], contact_force=cf.reshape(-1, 3)[:ncon],
+                    cfrc=cfrc, ft_torque=ft, gnorm=norms[0], rhs_norm=norms[1], hx_norm=norms[2], nefc=nefc)
 
     def eef(self):
         J, pos, mat = np.zeros(42), np.zeros(3), np.zeros(9)

@@ -598,3 +598,61 @@ def test_lane_per_link_formulation_matches_the_generic_tree(O, robot):
         assert np.abs(M[:nj, :nj] - e.M[:nj, :nj]).max() < 1e-10
         assert np.abs(bias[:nj] - e.bias[:nj]).max() < 1e-9
         assert np.abs(J - Jo).max() < 1e-12 and np.abs(site - pos).max() < 1e-12 and np.abs(Rs - mat).max() < 1e-12
+
+
+@pytest.mark.parametrize("scene", ["soft", "rigid", "cylinder"])
+def test_evaluate_at_the_oracle_optimum(O, scene):
+    """oracle_evaluate (the hook the device solve is judged with): at the oracle's own qacc the float64 gradient vanishes, the primal
+    cost is a minimum along random directions, and forces, cfrc and the F/T torque are those of the forward pass.  One arm joint
+    sits 0.02 rad past its lower limit and moves into it (the limit is moved, so the contacts stay), so a joint-limit row is active.
+    The env is left unchanged."""
+    import dataclasses
+    from rui_b200.abi import PackedModel
+    from rui_b200.model import SceneParams, build_model, cylinder_torso_params
+    params = cylinder_torso_params() if scene == "cylinder" else SceneParams(soft_torso=scene != "rigid")
+    rng = np.random.default_rng(7)
+    if scene == "rigid":  # fixed gains, the probe pressed onto the table
+        cfg = _cfg(CC_FIXED, seed=2)
+        e = O.OracleEnv(PackedModel(build_model(params)), cfg, 0)
+        e.reset()
+        for _ in range(250):
+            e.step(np.array([0, 0, -1, 0, 0, 0.0]))
+    else:
+        cfg = _cfg(CC_TRACK, seed=5, torso_solref_randomization=True, initial_probe_pos_randomization=True)
+        e = O.OracleEnv(PackedModel(build_model(params)), cfg, 0)
+        e.reset()
+        for _ in range(5):
+            e.step(rng.uniform(0, 1, 6))
+    q, v, w, t = e.get_state()
+    tau = e.tau
+    j = 3
+    rng_j = [list(r) for r in params.joint_range]
+    rng_j[j][0] = q[j] + 0.02
+    pk = PackedModel(build_model(dataclasses.replace(params, joint_range=tuple(tuple(r) for r in rng_j))))
+    e = O.OracleEnv(pk, cfg, 0)
+    e.reset()
+    v[j] = -0.3
+    e.set_state(q, v, w, t)
+    e.forward(tau)
+    a = e.qacc
+    c, d = e.contacts(), e.diag()
+    assert len(c["dist"]) >= (1 if scene == "rigid" else 10)
+    r = e.evaluate(a)
+    assert r["nefc"] == e.nefc and np.isfinite(r["grad"]).all()
+    lim = r["efc_type"] == 1
+    assert lim.sum() == 1 and r["efc_force"][lim][0] > 0  # the lower-limit row pushes the joint back
+    scale = 1 + r["rhs_norm"] + r["hx_norm"]
+    assert r["gnorm"] == pytest.approx(np.linalg.norm(r["grad"]), rel=1e-12) and r["gnorm"] <= 1e-9 * scale, (r["gnorm"], scale)
+    assert np.abs(r["contact_force"] - c["force"]).max() <= 1e-12 * max(1.0, np.abs(c["force"]).max())
+    assert np.abs(r["cfrc"] - d[0:3]).max() <= 1e-12 * max(1.0, np.abs(d[0:3]).max())
+    assert np.abs(r["ft_torque"] - d[3:6]).max() <= 1e-12 * max(1.0, np.abs(d[3:6]).max())
+    for _ in range(8):
+        dd = rng.standard_normal(e.nv) * 1e-3 * (1 + np.abs(a))
+        assert e.evaluate(a + dd)["cost"] > r["cost"] and e.evaluate(a - dd)["cost"] > r["cost"]
+    # elsewhere the gradient is M (a - a0) - J^T f, and the F/T torque follows qacc through the probe's acceleration
+    b = a + rng.standard_normal(e.nv) * 0.1
+    rb = e.evaluate(b)
+    assert np.abs(rb["grad"][:7] - (e.M @ (b - e.qacc_smooth))[:7]).max() > 1e-3 and np.abs(rb["ft_torque"] - d[3:6]).max() > 1e-6
+    # and the env is unchanged by the evaluations
+    assert np.array_equal(e.qacc, a) and np.array_equal(e.diag(), d) and np.array_equal(e.contacts()["force"], c["force"])
+    assert np.array_equal(e.evaluate(a)["efc_force"], r["efc_force"])
