@@ -21,7 +21,7 @@
  *     Use ONE stream for the stream-taking calls of a handle (or order your
  *     streams yourself).  usim_step_host works on a private stream: it waits
  *     (cudaStreamWaitEvent) for the last usim_reset / usim_step /
- *     usim_set_state issued on a caller's stream and synchronises its own
+ *     usim_forward / usim_set_state issued on a caller's stream and synchronises its own
  *     stream before returning, so the two kinds of call may be mixed freely.
  *   - no CPU fallback: usim_create fails if no sm_100-class device is present.
  *   - quaternions are (w,x,y,z) in qpos (MuJoCo), (x,y,z,w) where robosuite
@@ -170,6 +170,33 @@ int usim_reset(usim_handle* h, const uint8_t* mask_dev, float* obs_dev, void* st
 int usim_step(usim_handle* h, const float* act_dev, float* obs_dev, float* rew_dev,
               uint8_t* done_dev, float* term_obs_dev, int auto_reset, void* stream);
 
+/* Forward pass without stepping: MuJoCo's mj_forward at each selected env's
+ * live (qpos, qvel).  Replaces `sim.forward()` (ultrasound.py:431, and
+ * robosuite's `set_robot_joint_positions` after it writes qpos).
+ *   mask_dev  [num_envs] uint8, envs to evaluate (NULL: all)
+ *   ctrl_dev  [num_envs][7] float joint torques, clipped to ctrl_range as MuJoCo
+ *             clips a limited ctrl (NULL: zero, `data.ctrl` after mj_resetData;
+ *             UR5e: the seventh column is ignored)
+ *   obs_dev   [num_envs][19] float (may be NULL): the observation robosuite's
+ *             _get_observations(force_update=True) gives after sim.forward():
+ *             channels 0-8 and 12-18 from this pass (current kinematics, not
+ *             the site pose a step's observation carries), 9-11 from the task
+ *             record as it stands
+ *   qacc_dev  [num_envs][nv] float (may be NULL): the solved accelerations
+ * The constraint solve is warm-started from the env's qacc_warmstart row, with
+ * the reset forward pass's iteration cap (2 x solver_iterations) and the
+ * configured tolerance.  For the selected envs it refreshes usim_get_diag
+ * (torques = the clipped ctrl), usim_get_contacts and the contact record; every
+ * row of the other envs is left as it was.  It leaves the state (qpos, qvel,
+ * warm start, task record), the arm record (whose qfrc_smooth feeds the next
+ * step's warm-start shift: usim_get_arm_record keeps describing the last step
+ * or reset), the prepared reset states, the divergence / overflow counters and
+ * the done flags bit for bit as they were, so that the steps that follow run
+ * exactly as without the call.  Terminated envs are evaluated too and stay
+ * done.  A diverged pass reports zero forces and a finite observation, as a
+ * step does, and counts nothing.  Fails before the first usim_reset. */
+int usim_forward(usim_handle* h, const uint8_t* mask_dev, const float* ctrl_dev, float* obs_dev, float* qacc_dev, void* stream);
+
 /* Convenience for host callers (the end-to-end path of bench.py and of the
  * single-env robosuite-style API): HOST buffers; the H2D/D2H copies are done
  * inside the call, which synchronises the library's stream.  A buffer that is
@@ -232,7 +259,7 @@ int usim_set_contact_record(usim_handle* h, int enable);
  * it was last enabled.  A diverged env reports zero forces. */
 int usim_get_contact_forces(usim_handle* h, float* pos_dev, float* frame_dev, float* force_dev, void* stream);
 
-/* Per-env diagnostics of the last step, [num_envs][USIM_DIAG_DIM] float:
+/* Per-env diagnostics of the last forward pass (step, reset or usim_forward), [num_envs][USIM_DIAG_DIM] float:
  * 0-2 cfrc_ext[probe][-3:] (ultrasound.py:365), 3-5 ee torque (:369),
  * 6-8 eef pos, 9-12 eef quat xyzw, 13-19 joint torques, 20 solver iterations,
  * 21 solver gradient norm, 22 ncon (uncapped), 23 nefc, 24 preconditioner rebuilds, 25 line-search evaluations,
@@ -245,7 +272,8 @@ int usim_get_diag(usim_handle* h, float* diag_dev, void* stream);
  * controller output.  0-48 joint-space inertia M (7x7 row major), 49-55 qfrc_smooth of the arm, 56-62 clipped joint torques,
  * 63-104 grip-site Jacobian (rows 0-2 linear, 3-5 angular; 6x7), 105-125 hand-body linear Jacobian (3x7), 126-128 site position,
  * 129-137 site orientation (row major), 138-143 probe capsule end points, 144-146 / 147-167 F/T torque sensor: bias part and
- * linear map from the arm accelerations (3x7), 168-171 eef quaternion xyzw, 172-178 warm-start shift of the solver. */
+ * linear map from the arm accelerations (3x7), 168-171 eef quaternion xyzw, 172-178 warm-start shift of the solver.
+ * usim_forward does not write it: it keeps describing the last step or reset. */
 #define USIM_ARM_RECORD_DIM 180
 int usim_get_arm_record(usim_handle* h, float* rec_dev, void* stream);
 

@@ -23,6 +23,7 @@ SYMBOLS = {
     "usim_reset": (C.c_int, [_vp, _vp, _vp, _vp]),
     "usim_step": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _vp, C.c_int, _vp]),
     "usim_step_host": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _vp, C.c_int]),
+    "usim_forward": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _vp]),
     "usim_get_state": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _vp]),
     "usim_set_state": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _vp]),
     "usim_get_contacts": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _vp]),

@@ -102,11 +102,11 @@ __device__ __forceinline__ void osc_set_goal(const float* act, v3 site, const fl
   }
 }
 
-// mode: 0 = env step (controller runs), 1 = reset forward (ctrl = 0)
-// mode 0: env step (OSC torques from the action); mode 1: forward pass after a reset (ctrl = 0)
+// mode 0: env step (OSC torques from the action); mode 1: forward pass without a controller (after a reset, or usim_forward):
+// torques = the row `act` clipped to ctrl_range (nullptr: ctrl = 0), no warm-start shift
 // (q, qd: the arm joint positions / velocities of this env, in registers: the caller may have just written them to HBM itself)
 // policy_step: first physics substep of a control step -- the only one on which the OSC goal is set (robosuite Robot.control)
-// ts / ab: the env's task record and arm record; act: the env's action row
+// ts / ab: the env's task record and arm record; act: the env's action row (mode 0) or joint torque row [7] (mode 1)
 template <int NJ>
 __device__ __forceinline__ void arm_forward(int mode, bool policy_step, const float (&q)[7], const float (&qd)[7],
                                             const float* __restrict__ act, float* __restrict__ ts, float* __restrict__ ab) {
@@ -189,7 +189,7 @@ ARM_LOOP
   for (int j = 0; j < 7; j++) dx[j] = 0.f;
   if (mode == 1) {
 #pragma unroll
-    for (int j = 0; j < 7; j++) tau[j] = 0.f;
+    for (int j = 0; j < 7; j++) tau[j] = act && j < NJ ? fminf(fmaxf(act[j], -dm.ctrl[j]), dm.ctrl[j]) : 0.f; // (UR5e: slot 6 is inert)
   } else {
     float av[7];
     for (int i = 0; i < dm.adim; i++) av[i] = act[i];
@@ -380,6 +380,21 @@ __global__ void __launch_bounds__(64) arm_kernel(int n, const float* __restrict_
 #pragma unroll
   for (int j = 0; j < 7; j++) { q[j] = qpos[(size_t)env * QPAD + j]; qd[j] = qvel[(size_t)env * QPAD + j]; }
   arm_forward<NJ>(0, policy_step != 0, q, qd, act + (size_t)env * dm.adim, task + (size_t)env * USIM_TASK_DIM, armbuf + (size_t)env * ARMBUF);
+}
+
+// Arm part of usim_forward (mj_forward at the live state with the given joint torques), one thread per env: the arm record goes to
+// `armbuf`, the handle's forward buffer, never to the live record (its qfrc_smooth feeds the next step's warm-start shift).  Reads
+// qpos / qvel / task only.  ctrl: [n][7] joint torques, nullptr: zero; mask: envs to process (nullptr: all).
+template <int NJ>
+__global__ void __launch_bounds__(32) forward_arm_kernel(int n, const uint8_t* __restrict__ mask, const float* __restrict__ qpos,
+                                                         const float* __restrict__ qvel, const float* __restrict__ ctrl,
+                                                         float* __restrict__ task, float* __restrict__ armbuf) {
+  const int env = blockIdx.x * blockDim.x + threadIdx.x;
+  if (env >= n || (mask && !mask[env])) return;
+  float q[7], qd[7];
+#pragma unroll
+  for (int j = 0; j < 7; j++) { q[j] = qpos[(size_t)env * QPAD + j]; qd[j] = qvel[(size_t)env * QPAD + j]; }
+  arm_forward<NJ>(1, false, q, qd, ctrl ? ctrl + (size_t)env * 7 : nullptr, task + (size_t)env * USIM_TASK_DIM, armbuf + (size_t)env * ARMBUF);
 }
 
 // ---------------------------------------------------------------- reset (ultrasound.py:416-477, :749-887)

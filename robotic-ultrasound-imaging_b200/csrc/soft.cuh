@@ -376,6 +376,9 @@ struct SolveArgs {
   unsigned long long* trace;       // developer trace (USIM_TRACE): per env (start ns, end ns, SM id) of the launch, nullptr: off
   int* queue;                      // persistent launch (grid = resident CTAs): next launch slot, fetched with atomicAdd (nullptr: item = blockIdx.x + k gridDim.x)
   float* crec_out;                 // contact record [n][DEV_MAXC][CREC_DIM] (rows c < ncon), nullptr: recording off (usim_set_contact_record)
+  int fwd;                         // mode 1, live: usim_forward -- the observation takes its task channels from the record as it
+                                   // stands, and neither state rows nor the task record are stored
+  float* qacc_out;                 // usim_forward: [n][QPAD] the solution qacc, nullptr: not written
 };
 // one contact of the record: point (world), normal (geom1 -> geom2), world force on geom2 -- usim_get_contact_forces turns it into
 // MuJoCo's contact frame and frame-coordinate force
@@ -1578,6 +1581,10 @@ __global__ void __launch_bounds__(NT, MINB) solve_kernel(const SolveArgs a) {
   env_sync();
   // ------------------------------------------------------------------ contact record (opt-in, usim_set_contact_record)
   if (a.crec_out) record_contacts(w, a.crec_out + (size_t)env * DEV_MAXC * CREC_DIM, ncon, tid);
+  // usim_forward: K9 ran as after a reset, so the staged task channels hold initialised statistics; the observation takes them from
+  // the record as it stands (global memory: never stored in this mode), as a step's observation does
+  if (a.fwd && tid >= 9 && tid < 12)
+    w.orow[tid] = tid == 9 ? ts_g[USIM_TS_FZ_MEAN] - 5.f : tid == 10 ? ts_g[USIM_TS_DFZ] : ts_g[USIM_TS_VEL_MEAN] - 0.04f;
   if (mode != 2 && tid < USIM_OBS_DIM) { // this step's observation: the terminal one if a prepared reset state takes over below
     float* o = w.consume ? (a.tobs ? a.tobs + (size_t)env * USIM_OBS_DIM : nullptr) : obs_row;
     if (o) o[tid] = w.orow[tid];
@@ -1611,7 +1618,8 @@ __global__ void __launch_bounds__(NT, MINB) solve_kernel(const SolveArgs a) {
         tma_store_row(qv_g, w.hs, QPAD * 4);
         tma_store_row(wm_g, w.x, QPAD * 4);
       }
-      tma_store_row(ts_g, w.ts, USIM_TASK_DIM * 4);
+      if (!a.fwd) tma_store_row(ts_g, w.ts, USIM_TASK_DIM * 4);
+      else if (a.qacc_out) tma_store_row(a.qacc_out + (size_t)env * QPAD, w.x, QPAD * 4); // the solution (zero beyond nv)
       tma_store_commit_wait();
     }
   }

@@ -62,6 +62,8 @@ struct usim_handle {
   int64_t solve_tick = 0;
   // reset pipeline: two prepared reset states per env (slot k holds an episode number of parity k), made on a side stream
   float *slot_qpos = nullptr, *slot_task = nullptr, *slot_obs = nullptr, *prep_armbuf = nullptr;
+  // usim_forward, allocated on its first call: arm record ([n][ARMBUF]; the live one is left alone) and padded qacc rows ([n][QPAD])
+  float *fwd_armbuf = nullptr, *fwd_qacc = nullptr;
   int *req_list = nullptr, *req_cnt = nullptr; // [2][2 * 3n], [2]: request lists, double buffered by producer tick
   int64_t prod_tick = 0;
   bool slots_init = false;
@@ -324,7 +326,7 @@ int usim_destroy(usim_handle* h) {
   void* dev[] = {h->counters, h->qpos, h->qvel, h->warm, h->task, h->armbuf, h->diag, h->ncon, h->geom1, h->geom2, h->cdist, h->crec, h->ax4,
                  h->ps4, h->nb4, h->eq_pairs, h->d_act, h->d_obs, h->d_tobs, h->d_rew,
                  h->d_done, h->d_resetmask, h->bin_cnt, h->bin_items, h->order, h->queue, h->slot_qpos, h->slot_task, h->slot_obs, h->prep_armbuf,
-                 h->req_list, h->req_cnt};
+                 h->fwd_armbuf, h->fwd_qacc, h->req_list, h->req_cnt};
   for (void* p : dev) if (p) cudaFree(p);
   void* host[] = {h->h_act, h->h_obs, h->h_tobs, h->h_rew, h->h_done};
   for (void* p : host) if (p) cudaFreeHost(p);
@@ -501,6 +503,42 @@ int usim_reset(usim_handle* h, const uint8_t* mask_dev, float* obs_dev, void* st
   } else if (producer_end(h, s)) {
     return -1;
   }
+  return mark_state(h, s);
+}
+
+// padded qacc rows of usim_forward -> the caller's dense [n][nv] array, rows of the selected envs only
+__global__ void qacc_rows_kernel(int n, int nv, const uint8_t* __restrict__ mask, const float* __restrict__ src, float* __restrict__ dst) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n * nv) return;
+  const int e = i / nv, k = i - e * nv;
+  if (!mask || mask[e]) dst[i] = src[(size_t)e * QPAD + k];
+}
+
+// mj_forward at the live state: the arm pass into the forward buffer, then the solve kernel in forward mode (mode 1 as after a
+// reset, but warm-started from the live qacc_warmstart, the task record read and never written, no launch-order bins, no counters)
+int usim_forward(usim_handle* h, const uint8_t* mask_dev, const float* ctrl_dev, float* obs_dev, float* qacc_dev, void* stream) {
+  if (!h) return fail("usim_forward: null handle");
+  if (!h->slots_init) return fail("usim_forward: no state to evaluate before the first usim_reset");
+  if (activate(h)) return -1;
+  cudaStream_t s = (cudaStream_t)stream;
+  const int n = h->n;
+  if (!h->fwd_armbuf) CK(cudaMalloc((void**)&h->fwd_armbuf, (size_t)n * ARMBUF * sizeof(float)));
+  if (qacc_dev && !h->fwd_qacc) CK(cudaMalloc((void**)&h->fwd_qacc, (size_t)n * QPAD * sizeof(float)));
+  const int grid = (n + ARM_BLOCK - 1) / ARM_BLOCK;
+  if (h->narm == 7) forward_arm_kernel<7><<<grid, ARM_BLOCK, 0, s>>>(n, mask_dev, h->qpos, h->qvel, ctrl_dev, h->task, h->fwd_armbuf);
+  else forward_arm_kernel<6><<<grid, ARM_BLOCK, 0, s>>>(n, mask_dev, h->qpos, h->qvel, ctrl_dev, h->task, h->fwd_armbuf);
+  SolveArgs a = base_args(h, 1);
+  a.fwd = 1; a.armbuf = h->fwd_armbuf; a.mask = mask_dev; a.obs = obs_dev; a.qacc_out = qacc_dev ? h->fwd_qacc : nullptr;
+  a.counters = nullptr;
+  solve_kernel<<<n, NT, h->smem, s>>>(a);
+  h->launches += 2;
+  if (qacc_dev) { // (the solve kernel stores whole 16-byte aligned rows by TMA: a dense [n][nv] row is not aligned)
+    const int tot = n * h->nv;
+    qacc_rows_kernel<<<(tot + 255) / 256, 256, 0, s>>>(n, h->nv, mask_dev, h->fwd_qacc, qacc_dev);
+    h->launches += 1;
+  }
+  CK(cudaGetLastError());
+  if (h->crec_on && !mask_dev) h->crec_complete = true;
   return mark_state(h, s);
 }
 

@@ -150,6 +150,23 @@ class BatchedUltrasound:
                                             int(auto_reset), self._stream()))
         return self.obs, self.rew, self.done, self.term_obs
 
+    def forward(self, mask: Optional[torch.Tensor] = None, ctrl: Optional[torch.Tensor] = None, qacc: bool = False):
+        """``sim.forward()`` (MuJoCo ``mj_forward``) at the current state of the envs selected by ``mask`` (None: all), with joint
+        torques ``ctrl`` [N, 7] clipped to the actuator ranges (None: zero; UR5e: column 6 is ignored).  Refreshes :meth:`diag`,
+        :meth:`contacts` and :meth:`contact_forces` of the selected envs and writes their observation into ``self.obs`` (returned);
+        the state, the task record, :meth:`arm_record` and everything a later step reads are left as they were.  With
+        ``qacc=True`` returns ``(obs, qacc [N, nv])`` (rows of unselected envs are zero)."""
+        if mask is not None:
+            mask = mask.to(device=self.device, dtype=torch.uint8).contiguous()
+            assert mask.shape == (self.num_envs,), mask.shape
+        if ctrl is not None:
+            ctrl = torch.as_tensor(ctrl, dtype=torch.float32, device=self.device).contiguous()
+            assert ctrl.shape == (self.num_envs, 7), ctrl.shape
+        qa = torch.zeros(self.num_envs, self.nv, device=self.device) if qacc else None
+        with torch.cuda.device(self.device):
+            _lib.check(_lib.lib().usim_forward(self._h, _ptr(mask), _ptr(ctrl), _ptr(self.obs), _ptr(qa), self._stream()))
+        return (self.obs, qa) if qacc else self.obs
+
     def step_host(self, actions: np.ndarray, auto_reset: bool = True):
         """End-to-end call with HOST buffers (copies inside the library)."""
         a = np.ascontiguousarray(actions, dtype=np.float32)
@@ -360,10 +377,24 @@ class _Robot:
         return bool(np.any(~((rng[:, 0] + 0.1 < q) & (q < rng[:, 1] - 0.1))))
 
     def set_robot_joint_positions(self, jpos):
-        """ultrasound.py:462: overwrite the arm joint positions (velocities are left as they are, as in robosuite)."""
+        """ultrasound.py:462: overwrite the arm joint positions (velocities are left as they are), then ``sim.forward()``, as
+        robosuite does: eef pose, contacts and forces describe the new pose."""
         q = self._env.core.get_state()[0]
         q[0, :self.dof] = torch.as_tensor(np.asarray(jpos, dtype=np.float32), device=q.device)
         self._env.core.set_state(qpos=q)
+        self._env.sim.forward()
+
+
+class _Sim:
+    """``env.sim`` as far as the task code uses it: ``forward()`` (ultrasound.py:431)."""
+
+    def __init__(self, env: "Ultrasound"):
+        self._env = env
+
+    def forward(self):
+        """``sim.forward()`` with ``data.ctrl`` as MuJoCo keeps it: the torques last applied (diag[13:20]; zero after a reset)."""
+        core = self._env.core
+        core.forward(ctrl=core.diag()[:, 13:20])
 
 
 class Ultrasound:
@@ -443,6 +474,7 @@ class Ultrasound:
             initial_probe_pos_randomization=initial_probe_pos_randomization, deterministic_trajectory=deterministic_trajectory,
             seed=seed, ignore_done=ignore_done, scene_params=scene_params, record_contacts=True)
         self.robots = [_Robot(self)]
+        self.sim = _Sim(self)
         self.timestep = 0
         self.done = True
 
