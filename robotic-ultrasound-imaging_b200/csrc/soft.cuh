@@ -37,50 +37,22 @@
 // contact slots and aliased reduction zones the env image shrinks to 24.3 KB = 9 CTAs per SM, but the 9th needs <= 112 registers:
 // 120 regs / 8 CTAs 8.83 M env-steps/s, 112 / 9: 8.47 M, 96 / 9: 8.34 M, 96 / 8: 8.00 M -- the register-capped schedule costs 5-9 %, the
 // extra CTA returns 4 %.  Three or four warps per env at 8 envs per SM (24 / 32 warps, 80 / 72 registers): 7.22 / 6.22 M against 7.82 M.
-// Fewer resident envs (USIM_SMEM_PAD): 7 / 6 / 5 CTAs per SM = 8.18 / 7.70 / 7.22 M.
+// Fewer resident envs (shared memory padded per CTA): 7 / 6 / 5 CTAs per SM = 8.18 / 7.70 / 7.22 M.
 #define NPAIR_MAX 544
 #define SLOT_OBS 20 // row pitch of a prepared observation (19 used)
-// Slider block of the preconditioner, D - W (D: diagonal, W: the pair couplings of the shell grid), inverted by a polynomial in
-// N = D^-1 W.  PREC3 = 0: second order, D^-1 (I + N).  PREC3 = 1: third order with Chebyshev weights, D^-1 (I + c (N + N^2)),
-// c = 4 / (4 - 3 rho^2): the cubic (1 - x) p(x) = 1 - T3(x / rho) / T3(1 / rho) deviates least from 1 on the spectrum [-rho, rho]
-// of N.  rho ~ 0.7 for this model (sum of a slider's pair D over its diagonal) -> c = 1.6; measured at 4096 envs:
-// second order 0.513 ms, c = 1.0 (plain Neumann) 0.513, 1.4: 0.485, 1.7: 0.483, 2.0: 0.488, 2.4: 0.506, 3.0: 0.578;
-// fourth order (three stencil passes, a0 (z0 + z1) + a2 (z2 + z3)): 0.488 ms vs 0.464 for the cubic -- not kept.
-// Round 2, after the rebuild policy (most solves keep the preconditioner of their warm start): the SECOND-order block does as well as the
-// cubic in iterations and saves a stencil pass -- PREC3 = 0: 0.428 ms / 5.73 iterations, PREC3 = 1 (c = 1.1): 0.442 / 5.79; Jacobi
-// (PREC_JACOBI): 0.473 / 7.05; weight 0.8 / 1.2 / 1.4 on the first-order term (PREC2_C): 0.441 / 0.449 / 0.503.
-#ifndef PREC3
-#define PREC3 0
-#endif
-// Re-measured on the final kernel of round 2 (calibrated probe, line-search tolerance 0.03; kernel ms / CG iterations): 0.9: 0.487 / 5.31,
-// 1.0: 0.479 / 5.32, 1.1: 0.480 / 5.33, 1.2: 0.479 / 5.34, 1.3: 0.483 / 5.37, 1.4: 0.483 / 5.41, 1.5: 0.485 / 5.45, 1.6: 0.486 / 5.50,
-// 1.8: 0.497 / 5.65 -- the optimum is a plateau from the plain Neumann series (1.0) to 1.2: the contact terms on the diagonal have
-// lowered the effective rho.
-#ifndef CHEB_C
-#define CHEB_C 1.1f
-#endif
-// Arm part of the warm start: the previous qacc shifted by M^-1 (qfrc_smooth_now - qfrc_smooth_previous), computed by the arm kernel
-// with the Cholesky factor it holds anyway.  A fresh action every step moves qfrc_smooth of the arm by the change of the controller
-// torque; without the shift the previous qacc is a poor start for the 7 arm unknowns (6.4 CG iterations with random actions, 4.0 with
-// a constant one).
-#ifndef ARM_SHIFT
-#define ARM_SHIFT 1
-#endif
-#ifndef WARP_SOLVE
-#define WARP_SOLVE 0 // 1: dense blocks of the preconditioner solved by one warp with shuffles (chol7_solve_warp2) instead of replicated in every thread.  Measured at 4096 envs: 0.441 ms vs 0.4245 ms replicated -- ~150 instead of ~290 instructions, but the 28 dependent shuffles are the longer chain and the kernel is latency bound: not kept.  Re-measured with the first stencil pass on the second warp (SPLIT_Z1): 0.5064 vs 0.4993 ms
-#endif
-#ifndef SPLIT_SOLVE
-#define SPLIT_SOLVE (WPE == 2 && PREC3 && !WARP_SOLVE) // 1: the first warp solves the dense blocks while the second runs the first stencil pass of the slider block for all sliders (instead of both warps doing both)
-#endif
-#ifndef SPLIT_DENSE
-#define SPLIT_DENSE 0 // 1 (needs WPE == 2, PREC3 == 0): the first warp solves the 7x7 arm block, the second the 6x6 torso block, one more barrier, instead of both warps solving both.  Measured: 0.4280 vs 0.4281 ms -- parity green, no gain, not shipped
-#endif
-#ifndef SPLIT_Z1
-#define SPLIT_Z1 (SPLIT_SOLVE || (WARP_SOLVE && WPE == 2 && PREC3)) // the first stencil pass belongs to the second warp alone
-#endif
-#ifndef NORESTART
-#define NORESTART 1 // 1: keep the Polak-Ribiere direction across a preconditioner rebuild (flexible CG: beta uses the previous pg, made with the previous preconditioner) instead of restarting; measured 0.464 ms vs 0.485 ms
-#endif
+// Solver choices (DESIGN.md §6 has the measurements of the alternatives that were built and rejected):
+// - Slider block of the preconditioner, D - W (D: diagonal, W: the pair couplings of the shell grid), inverted to second order in
+//   N = D^-1 W: D^-1 (I + N), one stencil pass.  Since the rebuild policy (most solves keep the preconditioner of their warm start)
+//   it does as well in iterations as the third-order block with Chebyshev weights, which costs a second pass (round 2: 0.428 ms /
+//   5.73 iterations against 0.442 / 5.79); Jacobi (no pass): 0.473 / 7.05.
+// - The dense 7x7 arm and 6x6 torso blocks are solved by every thread: one warp solving them with shuffles runs ~150 instead of
+//   ~290 instructions, but its 28 dependent shuffles are the longer chain in a latency-bound kernel (0.441 ms against 0.4245 ms).
+// - The Polak-Ribiere direction is kept across a preconditioner rebuild (flexible CG: beta uses the previous pg, made with the
+//   previous preconditioner) instead of restarting: 0.464 ms against 0.485 ms.
+// - Arm part of the warm start: the previous qacc shifted by M^-1 (qfrc_smooth_now - qfrc_smooth_previous), computed by the arm kernel
+//   with the Cholesky factor it holds anyway.  A fresh action every step moves qfrc_smooth of the arm by the change of the controller
+//   torque; without the shift the previous qacc is a poor start for the 7 arm unknowns (6.4 CG iterations with random actions, 4.0
+//   with a constant one).
 #ifndef LS_TOL
 #define LS_TOL 0.03f // line search: stop when |phi'| has dropped by this factor.  An inexact search is enough for nonlinear CG (the
                      // converged solution does not depend on it, only the path).  Measured at 4096 envs on the final kernel of round 2
@@ -136,7 +108,7 @@ struct __align__(16) WS {
   // landing zones of the warp reductions, one per call site, one row per warp (readers add the rows in a fixed order: rd())
   float r3[WPE][24], rg[WPE][16], rp[WPE][16], rq[WPE][8], rl[2][WPE][4], rb1[WPE][24], rb2[WPE][24], rb3[WPE][24];
   float lsign[7], lD[7], laref[7];
-  float yS[8];                                         // torso part of P^-1 grad (world frame), warp 0 -> all threads
+  float spare[8];                                      // unused; keeps the later fields at their offsets (solve_kernel's code as measured)
   float Dt, areft;
   int ncon, okf;
   int consume;                                         // this env's episode ended and a prepared reset slot takes over (K9 -> all threads)
@@ -144,9 +116,7 @@ struct __align__(16) WS {
   int cnt[2][WPE];                                     // cross-warp prefix of the contact compaction (double buffered)
   float orow[SLOT_OBS];                                // observation row of this step (K9, thread 0) -> written out as ONE coalesced row
 };
-#ifndef SKIP_SMEM_ASSERT
 static_assert(sizeof(WS) + 1024 <= 233472 / MINB, "WS must leave room for MINB CTAs per SM");
-#endif
 static_assert(2 * QPAD >= NPAIR_MAX + 1, "pg|s double as the pair scratch of K3");
 
 __device__ __forceinline__ void env_sync() {
@@ -310,34 +280,6 @@ __device__ __forceinline__ bool chol7_warp2(float* A0, float* A1, int lane) {
     if (act && k <= r) A[r * 7 + k] = row[k];
   return ok;
 }
-// x <- (L L^T)^-1 b for TWO factors written by chol7_warp2, at once, by one warp: lane r (0..6) holds entry r of the right-hand side of
-// A0, lane 8 + r that of A1; the solution entry comes back in the same lane.  Column-oriented substitution: one broadcast shuffle and
-// one FMA per column (28 shuffles in all) instead of the ~290 replicated, fully unrolled instructions of chol7_solve<7> + <6> in every
-// thread -- the loop body of the solver has to fit the 32 KB instruction cache.
-__device__ __forceinline__ float chol7_solve_warp2(const float* A0, const float* A1, float b, int lane) {
-  const int base = lane & 8, r = lane & 7;
-  const float* A = base ? A1 : A0;
-  const bool act = lane < 16 && r < 7;
-  float Lr[7], Lc[7]; // row r of L left of the diagonal, column r below it (zero elsewhere: no predicates in the loops)
-#pragma unroll
-  for (int k = 0; k < 7; k++) {
-    Lr[k] = (act && k < r) ? A[r * 7 + k] : 0.f;
-    Lc[k] = (act && k > r) ? A[k * 7 + r] : 0.f;
-  }
-  const float dinv = act ? A[r * 7 + r] : 1.f;
-  if (!act) b = 0.f;
-#pragma unroll
-  for (int j = 0; j < 7; j++) { // L y = b
-    if (r == j) b *= dinv;
-    b -= Lr[j] * __shfl_sync(0xffffffffu, b, base + j);
-  }
-#pragma unroll
-  for (int j = 6; j >= 0; j--) { // L^T x = y
-    if (r == j) b *= dinv;
-    b -= Lc[j] * __shfl_sync(0xffffffffu, b, base + j);
-  }
-  return b;
-}
 
 // Launch slots are ordered longest-solve-first: every launch files its envs into NBIN bins by the number of CG iterations they
 // took; the arm kernel of the next physics step flattens the bins (highest first) into `order`, and CTA j of the next solve launch
@@ -480,13 +422,7 @@ __global__ void __launch_bounds__(NT, MINB) solve_kernel(const SolveArgs a) {
   for (int i = nv + tid; i < QPAD; i += NT) w.x[i] = 0.f; // the solver vectors are zero beyond nv
   if (tid < 7) {
     w.qdarm[tid] = w.hs[tid];
-#if ARM_SHIFT
-#ifdef ARM_SHIFT_SCALE // developer knob: damped shift (in contact M^-1 over-estimates the response of the arm)
-    if (mode != 1) w.x[tid] += ARM_SHIFT_SCALE * w.ab[AB_DX + tid];
-#else
     if (mode != 1) w.x[tid] += w.ab[AB_DX + tid]; // warm start of the arm follows the change of its applied force (arm kernel)
-#endif
-#endif
   }
   float quat[4] = {1, 0, 0, 0};
   if (dm.soft) {
@@ -918,65 +854,9 @@ __global__ void __launch_bounds__(NT, MINB) solve_kernel(const SolveArgs a) {
     // (fp32 floor of the gradient is ~eps * (|Hx| + |rhs|): the terms that cancel in it)
     gnorm = sqrtf(rd(w.rp, 10));
     if (gnorm <= dm.tol * (1.f + rhsn + hxn)) return false;
-#if WARP_SOLVE
-    // dense blocks: the first warp solves both at once (arm 7x7 in lanes 0-6, torso 6x6 in lanes 8-13); the arm part goes straight to
-    // pg, the torso part (world frame) to yS for everybody; the other warp goes ahead with the stencil pass, which needs neither
-    if (wrp == 0) {
-      const int k = lane & 7;
-      float rhs = 0.f;
-      if (lane < 7) rhs = w.grad[lane];
-      else if (dm.soft && lane >= 8 && lane < 11) // gd[7+k] - (m R t[0:3] + t[3:6])_k
-        rhs = w.grad[7 + k] - (mp * (w.R[3 * k] * rd(w.rp, 0) + w.R[3 * k + 1] * rd(w.rp, 1) + w.R[3 * k + 2] * rd(w.rp, 2)) + rd(w.rp, 3 + k));
-      else if (dm.soft && lane >= 11 && lane < 14) // (R gd[10:13])_k - t[6:9]_k
-        rhs = w.R[3 * (k - 3)] * w.grad[10] + w.R[3 * (k - 3) + 1] * w.grad[11] + w.R[3 * (k - 3) + 2] * w.grad[12] - rd(w.rp, 3 + k);
-      const float sol = chol7_solve_warp2(w.Pa, w.Sf, rhs, lane);
-      if (lane < 7) w.pg[lane] = sol;
-      else if (lane >= 8 && lane < 14) w.yS[k] = dm.soft ? sol : 0.f;
-    }
-    float b[6] = {0, 0, 0, 0, 0, 0};
-#else
     float y[6] = {0, 0, 0, 0, 0, 0};
     v3 yl = mk(0, 0, 0), yb = mk(0, 0, 0);
     float b[6] = {0, 0, 0, 0, 0, 0};
-#if SPLIT_DENSE
-    if (wrp == 0) { // arm block
-      float ga[7], ya[7];
-#pragma unroll
-      for (int j = 0; j < 7; j++) { ga[j] = w.grad[j]; ya[j] = ga[j]; }
-      chol7_solve<7>(w.Pa, ya);
-      if (tid == 0) {
-#pragma unroll
-        for (int j = 0; j < 7; j++) { w.pg[j] = ya[j]; b[0] += ga[j] * ya[j]; }
-      }
-    } else { // torso block (world frame), for everybody through yS
-      if (dm.soft) {
-        float gt[6], t9[9];
-#pragma unroll
-        for (int k = 0; k < 6; k++) gt[k] = w.grad[7 + k];
-#pragma unroll
-        for (int k = 0; k < 9; k++) t9[k] = rd(w.rp, k);
-        v3 tv = mp * mv(R, ld3(t9)) + ld3(t9 + 3), gw = mv(R, mk(gt[3], gt[4], gt[5])) - ld3(t9 + 6);
-        y[0] = gt[0] - tv.x; y[1] = gt[1] - tv.y; y[2] = gt[2] - tv.z; y[3] = gw.x; y[4] = gw.y; y[5] = gw.z;
-        chol7_solve<6>(w.Sf, y);
-        yb = mtv(R, mk(y[3], y[4], y[5])); // back to the body frame
-        if (lane == 0) {
-          w.pg[7] = y[0]; w.pg[8] = y[1]; w.pg[9] = y[2]; w.pg[10] = yb.x; w.pg[11] = yb.y; w.pg[12] = yb.z;
-          b[0] += gt[0] * y[0] + gt[1] * y[1] + gt[2] * y[2] + gt[3] * yb.x + gt[4] * yb.y + gt[5] * yb.z;
-        }
-      }
-      if (lane == 0) {
-#pragma unroll
-        for (int k = 0; k < 6; k++) w.yS[k] = y[k];
-      }
-    }
-    env_sync();
-#pragma unroll
-    for (int k = 0; k < 6; k++) y[k] = w.yS[k];
-    yl = mtv(R, mk(y[0], y[1], y[2]));
-#else
-#if SPLIT_SOLVE
-    if (wrp == 0) {
-#endif
     float gd[13]; // dense part of the gradient
 #pragma unroll
     for (int k = 0; k < 13; k++) gd[k] = w.grad[k];
@@ -1001,60 +881,7 @@ __global__ void __launch_bounds__(NT, MINB) solve_kernel(const SolveArgs a) {
         w.pg[7] = y[0]; w.pg[8] = y[1]; w.pg[9] = y[2]; w.pg[10] = yb.x; w.pg[11] = yb.y; w.pg[12] = yb.z;
         b[0] += gd[7] * y[0] + gd[8] * y[1] + gd[9] * y[2] + gd[10] * yb.x + gd[11] * yb.y + gd[12] * yb.z;
       }
-#if SPLIT_SOLVE
-#pragma unroll
-      for (int k = 0; k < 6; k++) w.yS[k] = y[k];
-#endif
     }
-#if SPLIT_SOLVE
-    } // (first warp)
-#endif
-#endif // SPLIT_DENSE
-#endif
-#if PREC3
-#if SPLIT_Z1
-    if (wrp == 1) { // (the whole pass by the second warp, while the first one solves)
-      PRAGMA_HOT_S
-      for (int i = lane; i < np; i += 32) {
-        const int4 e = pt.nb4[i];
-        float nb = w.Dp[e.x >> 16] * w.hs[13 + (e.x & 0x7fff)] + w.Dp[e.y >> 16] * w.hs[13 + (e.y & 0x7fff)] +
-                   w.Dp[e.z >> 16] * w.hs[13 + (e.z & 0x7fff)] + w.Dp[e.w >> 16] * w.hs[13 + (e.w & 0x7fff)];
-        w.pg[13 + i] = nb * w.dg[i];
-      }
-    }
-#else
-    PRAGMA_HOT_S
-    for (int i = tid; i < np; i += NT) {
-      const int4 e = pt.nb4[i];
-      float nb = w.Dp[e.x >> 16] * w.hs[13 + (e.x & 0x7fff)] + w.Dp[e.y >> 16] * w.hs[13 + (e.y & 0x7fff)] +
-                 w.Dp[e.z >> 16] * w.hs[13 + (e.z & 0x7fff)] + w.Dp[e.w >> 16] * w.hs[13 + (e.w & 0x7fff)];
-      w.pg[13 + i] = nb * w.dg[i];
-    }
-#endif
-#endif
-#if WARP_SOLVE || PREC3
-    env_sync();
-#endif
-#if SPLIT_SOLVE
-    // the dense solution of the first warp, for everybody
-#pragma unroll
-    for (int k = 0; k < 6; k++) y[k] = w.yS[k];
-    yl = mtv(R, mk(y[0], y[1], y[2]));
-#endif
-#if WARP_SOLVE
-    float y[6];
-#pragma unroll
-    for (int k = 0; k < 6; k++) y[k] = w.yS[k];
-    const v3 yl = mtv(R, mk(y[0], y[1], y[2]));
-    if (tid < 13) { // dense part of pg (the torso rotation goes back to the body frame) and its share of grad.pg
-      float pgk;
-      if (tid < 7) pgk = w.pg[tid];
-      else if (tid < 10) pgk = y[0] * (tid == 7) + y[1] * (tid == 8) + y[2] * (tid == 9);
-      else { const int c = tid - 10; pgk = w.R[c] * y[3] + w.R[3 + c] * y[4] + w.R[6 + c] * y[5]; }
-      if (tid >= 7) w.pg[tid] = dm.soft ? pgk : 0.f;
-      if (tid < 7 || dm.soft) b[0] += w.grad[tid] * pgk;
-    }
-#endif
     PRAGMA_HOT_S
     for (int i = tid; i < np; i += NT) {
       float g = w.grad[13 + i];
@@ -1065,26 +892,10 @@ __global__ void __launch_bounds__(NT, MINB) solve_kernel(const SolveArgs a) {
         by += w.sk[0][cs] * y[0] + w.sk[1][cs] * y[1] + w.sk[2][cs] * y[2] + w.sc[0][cs] * y[3] + w.sc[1][cs] * y[4] + w.sc[2][cs] * y[5];
       // slider block D - W (W: the pair couplings) inverted to second order, D^-1 + D^-1 W D^-1: hs holds D^-1 grad
       const int4 e = pt.nb4[i];
-#if PREC3
-      // third order with Chebyshev weights: z0 + c (z1 + z2), z1 = D^-1 W z0 (in pg), z2 = D^-1 W z1
-      float nb = w.Dp[e.x >> 16] * w.pg[13 + (e.x & 0x7fff)] + w.Dp[e.y >> 16] * w.pg[13 + (e.y & 0x7fff)] +
-                 w.Dp[e.z >> 16] * w.pg[13 + (e.z & 0x7fff)] + w.Dp[e.w >> 16] * w.pg[13 + (e.w & 0x7fff)];
-      float p = w.hs[13 + i] + CHEB_C * (w.pg[13 + i] + nb * w.dg[i]) - by * w.dg[i];
-      w.hs[13 + i] = p; // neighbours read pg in this pass, not hs
-#else
-#ifdef PREC_JACOBI // developer knob: diagonal slider block (no stencil pass at all)
-      float nb = 0.f;
-#else
       float nb = w.Dp[e.x >> 16] * w.hs[13 + (e.x & 0x7fff)] + w.Dp[e.y >> 16] * w.hs[13 + (e.y & 0x7fff)] +
                  w.Dp[e.z >> 16] * w.hs[13 + (e.z & 0x7fff)] + w.Dp[e.w >> 16] * w.hs[13 + (e.w & 0x7fff)];
-#endif
-#ifdef PREC2_C // developer knob: weight of the first-order term of the second-order slider block
-      float p = w.hs[13 + i] + (PREC2_C * nb - by) * w.dg[i];
-#else
       float p = w.hs[13 + i] + (nb - by) * w.dg[i];
-#endif
       w.pg[13 + i] = p;
-#endif
       b[0] += g * p; b[2] += p;
       b[3] += mp * ah.x * p; b[4] += mp * ah.y * p; b[5] += mp * ah.z * p;
     }
@@ -1345,36 +1156,20 @@ __global__ void __launch_bounds__(NT, MINB) solve_kernel(const SolveArgs a) {
     const bool changed = rd(w.rg, 12) >= (it < REBUILD_LATE ? (float)REBUILD_MIN : 1.f);
     hxn = sqrtf(rd(w.rg, 13));
     if (init) rhsn = sqrtf(rd(w.rg, 14));
-    bool restart = init;
     // soft scene: rebuild when the active set moved; rigid scene (7 unknowns): exact Hessian every iteration = Newton
     if (init || (changed && rebuilds < dm.max_rebuilds) || (!dm.soft && ncon > 0)) {
       build_precond();
       rebuilds += init ? 0 : 1;
-      restart = init || !NORESTART;
     }
     if (!precond()) break;
     const float gpo = rd(w.rp, 9), gpn = rd(w.rq, 0); // grad.pg with the previous pg (Polak-Ribiere) and with the new one
-#ifdef RESTART_EVERY // developer knob: periodic steepest-descent restart of the nonlinear CG (measured, every 5 / 8 / 12 iterations: 7.82 / 7.68 / 7.86 M against 7.90 M without: long solves are not stalled directions)
-    if (it > 0 && it % RESTART_EVERY == 0) restart = true;
-#endif
-#ifdef BETA_FR // developer knob: Fletcher-Reeves instead of Polak-Ribiere+ (measured: 6.93 instead of 5.79 iterations, 0.655 vs 0.441 ms)
-    float beta = restart ? 0.f : gpn / fmaxf(gpg, 1e-30f);
-#else
-    float beta = restart ? 0.f : fmaxf(0.f, (gpn - gpo) / fmaxf(gpg, 1e-30f));
-#endif
+    // a rebuild keeps the direction: only the first iteration is steepest descent
+    float beta = init ? 0.f : fmaxf(0.f, (gpn - gpo) / fmaxf(gpg, 1e-30f));
     gpg = gpn;
 #pragma unroll
     for (int k = 0; k < 4; k++) S4[k] = -rd(w.rq, 2 + k) + beta * S4[k];
     PRAGMA_HOT_S
-#if PREC3
-    for (int i = tid; i < nv; i += NT) {
-      float p = i >= 13 ? w.hs[i] : w.pg[i];
-      w.pg[i] = p;
-      w.s[i] = -p + beta * w.s[i];
-    }
-#else
     for (int i = tid; i < nv; i += NT) w.s[i] = -w.pg[i] + beta * w.s[i];
-#endif
     env_sync();
   }
 

@@ -47,12 +47,12 @@ struct usim_handle {
   float4 *ax4 = nullptr, *ps4 = nullptr; // (axis, dof_invweight0), (rest position, body_invweight0)
   int4* nb4 = nullptr;                   // packed neighbour / pair stencil
   int2* eq_pairs = nullptr;
-  // staging for the host-buffer path
+  // staging for the host-buffer path: page-locked buffers, the device aliases of the output ones, and the actions on the device
   float *h_act = nullptr, *h_obs = nullptr, *h_rew = nullptr, *h_tobs = nullptr;
   uint8_t* h_done = nullptr;
-  float *d_act = nullptr, *d_obs = nullptr, *d_rew = nullptr, *d_tobs = nullptr;
-  uint8_t* d_done = nullptr;
-  uint8_t* d_resetmask = nullptr;
+  float *map_obs = nullptr, *map_rew = nullptr, *map_tobs = nullptr;
+  uint8_t* map_done = nullptr;
+  float* d_act = nullptr;
   // launch order of the solve kernel (longest solve first): bins filled by launch T, flattened by the arm kernel of launch T + 1
   int *bin_cnt = nullptr, *bin_items = nullptr, *order = nullptr; // [2][NBIN], [2][NBIN][n], [n]
   int* queue = nullptr;  // work queue of a persistent step launch (next launch slot)
@@ -72,11 +72,10 @@ struct usim_handle {
   bool ev_prep_valid[2] = {false, false};
   cudaStream_t own_stream = nullptr;
   cudaEvent_t ev_state = nullptr; // recorded on the caller's stream after every state-mutating call: usim_step_host waits on it
-  bool ev_state_valid = false, timing = false, arm_thread = false, host_copy = false;
+  bool ev_state_valid = false, timing = false, arm_thread = false;
   std::vector<std::pair<cudaEvent_t, cudaEvent_t>> pending;
   int64_t launches = 0, timed_launches = 0;
   double timed_ms = 0.0;
-  size_t smem = 0;
 };
 
 static usim_handle* g_active = nullptr; // handle whose DevModel currently sits in the constant block
@@ -249,14 +248,12 @@ int usim_create(const usim_model* m, const usim_config* c, int device, usim_hand
   CKH(cudaMallocHost((void**)&h->h_tobs, N * USIM_OBS_DIM * sizeof(float)));
   CKH(cudaMallocHost((void**)&h->h_rew, N * sizeof(float)));
   CKH(cudaMallocHost((void**)&h->h_done, N));
+  // the solve kernel writes the output staging buffers through these (UVA maps every page-locked allocation)
+  CKH(cudaHostGetDevicePointer((void**)&h->map_obs, h->h_obs, 0));
+  CKH(cudaHostGetDevicePointer((void**)&h->map_tobs, h->h_tobs, 0));
+  CKH(cudaHostGetDevicePointer((void**)&h->map_rew, h->h_rew, 0));
+  CKH(cudaHostGetDevicePointer((void**)&h->map_done, h->h_done, 0));
   CKH(cudaMalloc((void**)&h->d_act, N * USIM_MAX_ACTION * sizeof(float)));
-  CKH(cudaMalloc((void**)&h->d_obs, N * USIM_OBS_DIM * sizeof(float)));
-  CKH(cudaMalloc((void**)&h->d_tobs, N * USIM_OBS_DIM * sizeof(float)));
-  CKH(cudaMalloc((void**)&h->d_rew, N * sizeof(float)));
-  CKH(cudaMalloc((void**)&h->d_done, N));
-  CKH(cudaMalloc((void**)&h->d_resetmask, N));
-  CKH(cudaMemset(h->d_obs, 0, N * USIM_OBS_DIM * sizeof(float)));
-  CKH(cudaMemset(h->d_tobs, 0, N * USIM_OBS_DIM * sizeof(float)));
   CKH(cudaEventCreateWithFlags(&h->ev_state, cudaEventDisableTiming));
   CKH(cudaStreamCreateWithFlags(&h->own_stream, cudaStreamNonBlocking));
   {
@@ -291,8 +288,6 @@ int usim_create(const usim_model* m, const usim_config* c, int device, usim_hand
     CKH(cudaEventCreateWithFlags(&h->ev_prep[1], cudaEventDisableTiming));
   }
   if (const char* at = getenv("USIM_ARM_THREAD")) h->arm_thread = atoi(at) != 0;
-  if (const char* hc = getenv("USIM_HOST_COPY")) h->host_copy = atoi(hc) != 0;
-  h->smem = sizeof(WS);
   if (const char* tp = getenv("USIM_TRACE")) { // developer knob: the last step launch's per-env timeline is written to this file at destroy
     h->trace_path = tp;
     CKH(cudaMalloc((void**)&h->trace, (size_t)h->n * 3 * sizeof(unsigned long long)));
@@ -303,8 +298,7 @@ int usim_create(const usim_model* m, const usim_config* c, int device, usim_hand
     if (atoi(pg) != 0 && cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, solve_kernel, NT, sizeof(WS)) == cudaSuccess && per_sm > 0)
       h->step_grid = std::min(h->n, per_sm * prop.multiProcessorCount);
   }
-  if (const char* pad = getenv("USIM_SMEM_PAD")) h->smem += (size_t)atoi(pad); // developer knob: trade resident CTAs for L1 capacity
-  CKH(cudaFuncSetAttribute(solve_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->smem));
+  CKH(cudaFuncSetAttribute(solve_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(WS)));
   CKH(cudaDeviceSynchronize());
   *out = h;
   return 0;
@@ -324,8 +318,7 @@ int usim_destroy(usim_handle* h) {
   }
   for (auto& p : h->pending) { cudaEventDestroy(p.first); cudaEventDestroy(p.second); }
   void* dev[] = {h->counters, h->qpos, h->qvel, h->warm, h->task, h->armbuf, h->diag, h->ncon, h->geom1, h->geom2, h->cdist, h->crec, h->ax4,
-                 h->ps4, h->nb4, h->eq_pairs, h->d_act, h->d_obs, h->d_tobs, h->d_rew,
-                 h->d_done, h->d_resetmask, h->bin_cnt, h->bin_items, h->order, h->queue, h->slot_qpos, h->slot_task, h->slot_obs, h->prep_armbuf,
+                 h->ps4, h->nb4, h->eq_pairs, h->d_act, h->bin_cnt, h->bin_items, h->order, h->queue, h->slot_qpos, h->slot_task, h->slot_obs, h->prep_armbuf,
                  h->fwd_armbuf, h->fwd_qacc, h->req_list, h->req_cnt};
   for (void* p : dev) if (p) cudaFree(p);
   void* host[] = {h->h_act, h->h_obs, h->h_tobs, h->h_rew, h->h_done};
@@ -413,7 +406,7 @@ static int producer_end(usim_handle* h, cudaStream_t s) {
   SolveArgs a = base_args(h, 1);
   a.prep = 1; a.armbuf = h->prep_armbuf; a.prep_items = list; a.prep_n = cnt;
   a.diag = nullptr; a.ncon_out = nullptr; a.geom1_out = nullptr; a.geom2_out = nullptr; a.dist_out = nullptr; a.crec_out = nullptr;
-  solve_kernel<<<PREP_GRID, NT, h->smem, h->prep_stream>>>(a);
+  solve_kernel<<<PREP_GRID, NT, sizeof(WS), h->prep_stream>>>(a);
   CK(cudaMemsetAsync(cnt, 0, sizeof(int), h->prep_stream));
   CK(cudaEventRecord(h->ev_prep[b], h->prep_stream));
   h->ev_prep_valid[b] = true;
@@ -463,7 +456,7 @@ static int launch_step(usim_handle* h, const float* act, float* obs, float* rew,
       CK(cudaEventCreate(&e0)); CK(cudaEventCreate(&e1));
       CK(cudaEventRecord(e0, s));
     }
-    solve_kernel<<<h->step_grid ? h->step_grid : n, NT, h->smem, s>>>(a);
+    solve_kernel<<<h->step_grid ? h->step_grid : n, NT, sizeof(WS), s>>>(a);
     if (timed) {
       CK(cudaEventRecord(e1, s));
       h->pending.emplace_back(e0, e1);
@@ -493,7 +486,7 @@ int usim_reset(usim_handle* h, const uint8_t* mask_dev, float* obs_dev, void* st
   RESET_LAUNCH(h, (n + 31) / 32, 32, s, n, mask_dev, h->qpos, h->qvel, h->warm, h->task, h->armbuf, nullptr, nullptr, list, cnt);
   SolveArgs a = base_args(h, 1);
   a.mask = mask_dev; a.obs = obs_dev;
-  solve_kernel<<<n, NT, h->smem, s>>>(a);
+  solve_kernel<<<n, NT, sizeof(WS), s>>>(a);
   h->launches += 2;
   CK(cudaGetLastError());
   if (h->crec_on && !mask_dev) h->crec_complete = true;
@@ -530,7 +523,7 @@ int usim_forward(usim_handle* h, const uint8_t* mask_dev, const float* ctrl_dev,
   SolveArgs a = base_args(h, 1);
   a.fwd = 1; a.armbuf = h->fwd_armbuf; a.mask = mask_dev; a.obs = obs_dev; a.qacc_out = qacc_dev ? h->fwd_qacc : nullptr;
   a.counters = nullptr;
-  solve_kernel<<<n, NT, h->smem, s>>>(a);
+  solve_kernel<<<n, NT, sizeof(WS), s>>>(a);
   h->launches += 2;
   if (qacc_dev) { // (the solve kernel stores whole 16-byte aligned rows by TMA: a dense [n][nv] row is not aligned)
     const int tot = n * h->nv;
@@ -575,62 +568,38 @@ int usim_step_host(usim_handle* h, const float* act, float* obs, float* rew, uin
   cudaStream_t s = h->own_stream;
   size_t N = (size_t)h->n;
   const size_t row = USIM_OBS_DIM * sizeof(float);
-  // Caller buffers that are page-locked are used directly; pageable ones go through the library's pinned staging buffers.
+  // A page-locked action array is copied from directly; a pageable one goes through the library's pinned staging buffer.
   const float* a_src = act;
   if (!is_pinned(act)) { memcpy(h->h_act, act, N * h->adim * sizeof(float)); a_src = h->h_act; }
-  float* r_dst = rew && is_pinned(rew) ? rew : h->h_rew;
-  uint8_t* d_dst = done && is_pinned(done) ? done : h->h_done;
-  // Observation rows -- and the terminal rows of the envs that finish in this step, typically ~N / episode length of them -- are
-  // written by the solve kernel STRAIGHT into page-locked host memory (one coalesced 76-byte row per env, posted PCIe writes that
-  // overlap the rest of the launch): no device->host copy of the 19-column array after the kernel, no second round trip for the
-  // terminal rows, and only the rows of finished envs are touched in `term_obs_host`.  (USIM_HOST_COPY=1: the copy-based path.)
-  float* o_host = obs && is_pinned(obs) ? obs : h->h_obs;
-  float* t_host = tobs && is_pinned(tobs) ? tobs : h->h_tobs;
-  float* o_dev = h->host_copy ? nullptr : (float*)mapped_alias(o_host);
-  float* t_dev = h->host_copy ? nullptr : (float*)mapped_alias(t_host);
-  float* r_dev = h->host_copy ? nullptr : (float*)mapped_alias(r_dst);     // reward and done flag of an env: two more posted writes
-  uint8_t* d_dev = h->host_copy ? nullptr : (uint8_t*)mapped_alias(d_dst);
-  const bool zero_copy = o_dev && t_dev && r_dev && d_dev;
+  // Observation rows, reward, done flag -- and the terminal rows of the envs that finish in this step, typically ~N / episode length
+  // of them -- are written by the solve kernel STRAIGHT into page-locked host memory (one coalesced 76-byte row per env, posted PCIe
+  // writes that overlap the rest of the launch): no device->host copy after the kernel, no second round trip for the terminal rows,
+  // and only the rows of finished envs are touched in `term_obs_host`.  A caller buffer with a device alias is written in place; any
+  // other goes through the library's staging buffer.
+  float* o_dev = (float*)mapped_alias(obs);
+  float* t_dev = (float*)mapped_alias(tobs);
+  float* r_dev = (float*)mapped_alias(rew);
+  uint8_t* d_dev = (uint8_t*)mapped_alias(done);
+  float* o_host = o_dev ? obs : h->h_obs;
+  float* t_host = t_dev ? tobs : h->h_tobs;
+  float* r_host = r_dev ? rew : h->h_rew;
+  uint8_t* d_host = d_dev ? done : h->h_done;
+  if (!o_dev) o_dev = h->map_obs;
+  if (!t_dev) t_dev = h->map_tobs;
+  if (!r_dev) r_dev = h->map_rew;
+  if (!d_dev) d_dev = h->map_done;
   // the private stream is ordered after the last state-mutating call made on a caller's stream (usim_reset / usim_step /
   // usim_set_state), and this call synchronises it before returning: the two kinds of call may be mixed freely
   if (h->ev_state_valid) CK(cudaStreamWaitEvent(s, h->ev_state, 0));
   CK(cudaMemcpyAsync(h->d_act, a_src, N * h->adim * sizeof(float), cudaMemcpyHostToDevice, s));
-  if (zero_copy) {
-    if (usim_step(h, h->d_act, o_dev, r_dev, d_dev, tobs ? t_dev : nullptr, auto_reset, s)) return -1;
-  } else {
-    if (usim_step(h, h->d_act, h->d_obs, h->d_rew, h->d_done, tobs ? h->d_tobs : nullptr, auto_reset, s)) return -1;
-    CK(cudaMemcpyAsync(o_host, h->d_obs, N * row, cudaMemcpyDeviceToHost, s));
-    CK(cudaMemcpyAsync(r_dst, h->d_rew, N * sizeof(float), cudaMemcpyDeviceToHost, s));
-    CK(cudaMemcpyAsync(d_dst, h->d_done, N, cudaMemcpyDeviceToHost, s));
-  }
+  if (usim_step(h, h->d_act, o_dev, r_dev, d_dev, tobs ? t_dev : nullptr, auto_reset, s)) return -1;
   CK(cudaStreamSynchronize(s));
   if (obs && o_host != obs) memcpy(obs, o_host, N * row);
-  if (rew && r_dst != rew) memcpy(rew, h->h_rew, N * sizeof(float));
-  if (done && d_dst != done) memcpy(done, h->h_done, N);
-  if (tobs && zero_copy) {
-    if (t_host != tobs) { // pageable caller array: the kernel wrote the finished envs' rows into the staging buffer
-      for (size_t e = 0; e < N; e++)
-        if (d_dst[e]) memcpy(tobs + e * USIM_OBS_DIM, t_host + e * USIM_OBS_DIM, row);
-    }
-  } else if (tobs) {
-    // copy-based path: fetch the rows of the finished envs alone; when many envs finish together (a common horizon) one copy of
-    // the whole array into the library's staging buffer is cheaper.  Either way ONLY the rows of finished envs are written.
-    size_t ndone = 0;
-    for (size_t e = 0; e < N; e++) ndone += d_dst[e] != 0;
-    if (ndone > 64) {
-      CK(cudaMemcpyAsync(h->h_tobs, h->d_tobs, N * row, cudaMemcpyDeviceToHost, s));
-      CK(cudaStreamSynchronize(s));
-      for (size_t e = 0; e < N; e++)
-        if (d_dst[e]) memcpy(tobs + e * USIM_OBS_DIM, h->h_tobs + e * USIM_OBS_DIM, row);
-    } else if (ndone > 0) {
-      for (size_t e = 0; e < N; e++)
-        if (d_dst[e]) CK(cudaMemcpyAsync(t_host + e * USIM_OBS_DIM, h->d_tobs + e * USIM_OBS_DIM, row, cudaMemcpyDeviceToHost, s));
-      CK(cudaStreamSynchronize(s));
-      if (t_host != tobs) {
-        for (size_t e = 0; e < N; e++)
-          if (d_dst[e]) memcpy(tobs + e * USIM_OBS_DIM, h->h_tobs + e * USIM_OBS_DIM, row);
-      }
-    }
+  if (rew && r_host != rew) memcpy(rew, r_host, N * sizeof(float));
+  if (done && d_host != done) memcpy(done, d_host, N);
+  if (tobs && t_host != tobs) { // the kernel wrote the finished envs' rows into the staging buffer
+    for (size_t e = 0; e < N; e++)
+      if (d_host[e]) memcpy(tobs + e * USIM_OBS_DIM, t_host + e * USIM_OBS_DIM, row);
   }
   return 0;
 }
